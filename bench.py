@@ -2,7 +2,7 @@
 """bench.py — bases evaluated per second by the extreme-point enumeration path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--m 12 --n 40 --seed 1]
-                    [--algo auto|independent|shared] [--impl ours|reference]
+                    [--algo auto|independent|shared] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one complete enumeration of all C(n, m) bases of one synthetic dense
 LP (default: BASELINE.json's roofline headline, m=12, n=40 -> 5 586 853 480
@@ -24,6 +24,10 @@ Printed JSON line (rank 0):
             probe, nominal 148 SM x 64 lanes x 2 x f_max) (MEASURED_PEAKS.json
             carries no FP64 figure)
   cpu_baseline  the CPU oracle on this box's host cores on a bounded sample
+
+--dump-outputs DIR writes the last timed step's result records (status, best_rank, basis,
+x_B, objective, counts: one row per record) as float64 DIR/<name>.npy: the merged record
+of all ranks for the GPU arm, one record per sampled window for --impl reference.
 
 --impl reference times the CPU arm only (the reference's EnumerationSolver is
 an unimplemented stub and its building blocks need Eigen, which is not on the
@@ -120,15 +124,31 @@ def cpu_baseline(A, b, c, mx, m, n, budget_ranks, threads):
     from oracle import enumcpu
     total = binom(n, m)
     wins = cpu_sample_windows(total, budget_ranks)
-    ranks, secs = 0, 0.0
+    ranks, secs, results = 0, 0.0, []
     for (a, e) in wins:
         t = time.perf_counter()
-        enumcpu.solve(A, b, c, mx, n_threads=threads, rank_begin=a, rank_end=e)
+        results.append(enumcpu.solve(A, b, c, mx, n_threads=threads, rank_begin=a, rank_end=e)[0])
         secs += time.perf_counter() - t
         ranks += e - a
     desc = (f"full range of {total} ranks" if len(wins) == 1 else
             f"{ranks} of {total} ranks: prefix [0,{wins[0][1]}) + 8 windows of {wins[1][1] - wins[1][0]} ranks")
-    return ranks / secs, desc, ranks, secs
+    return ranks / secs, desc, ranks, secs, results
+
+
+def dump_outputs(out_dir, results, m):
+    """The result records of a step, one row per record, as float64 .npy files (ranks and counts are below 2^53,
+    so exact).  The workload is seeded: the same arguments give the same inputs, so two builds compare file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        "status": [r.status for r in results],
+        "best_rank": [r.best_rank for r in results],
+        "basis": [list(r.basis)[:m] for r in results],
+        "x_B": [list(r.x_B)[:m] for r in results],
+        "objective": [r.objective for r in results],
+        "counts": [[r.n_bases, r.n_singular, r.n_infeasible, r.n_feasible] for r in results],
+    }
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def reference_code_rate(A, b, c, mx, m, n, threads, seconds=4.0):
@@ -183,7 +203,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cpu-ranks", type=int, default=120_000_000, help="ranks in the CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result records of the last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -203,10 +227,12 @@ def main():
         budget = max(args.cpu_ranks // 4, 1_000_000)
         for _ in range(args.warmup):
             cpu_baseline(A, b, c, mx, m, n, budget // 8, threads)
-        t_ranks, t_secs, desc = 0, 0.0, ""
+        t_ranks, t_secs, desc, step_results = 0, 0.0, "", []
         for _ in range(args.steps):
-            _, desc, r, s = cpu_baseline(A, b, c, mx, m, n, budget, threads)
+            _, desc, r, s, step_results = cpu_baseline(A, b, c, mx, m, n, budget, threads)
             t_ranks += r; t_secs += s
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, step_results, m)     # one record per sampled window
         v = t_ranks / t_secs
         ref_code = reference_code_rate(A, b, c, mx, m, n, threads)
         kind, sample_note = "port", ("the reference's EnumerationSolver is a stub and Eigen is absent, so the arm is the "
@@ -329,7 +355,9 @@ def main():
     # show up as 2 ms outliers in the host-timed e2e steps below
     clocks = sampler.stop() if rank == 0 else None
     own_bases = _abi.Partial.from_buffer_copy(part.cpu().numpy().tobytes()).n_bases
-    res = edist.merge_records(gathered.cpu().numpy().tobytes(), world)
+    res = edist.merge_records(gathered.cpu().numpy().tobytes(), world)     # the last timed step's records, merged
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [res], m)
     value = total * args.steps / timed_s
 
     # ---- end to end through the public host-buffer API ------------------
@@ -482,7 +510,7 @@ def main():
     }
     if world == 1 and not args.no_cpu_baseline:
         threads = os.cpu_count() or 1
-        v, desc, _, _ = cpu_baseline(A, b, c, mx, m, n, args.cpu_ranks, threads)
+        v, desc, _, _, _ = cpu_baseline(A, b, c, mx, m, n, args.cpu_ranks, threads)
         out["cpu_baseline"] = {"value": v, "unit": "bases/s", "cores": threads, "kind": "port",
                                "sample": desc + "; Eigen-free oracle port (the reference path is a stub and Eigen is absent)"}
     print(json.dumps(out), flush=True)
