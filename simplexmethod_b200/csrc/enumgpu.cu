@@ -476,6 +476,10 @@ static int resolve(const enumgpu_problem* p, const enumgpu_options* o, Resolved*
     if (r->rule != ENUMGPU_PIVOT_ABSOLUTE && r->rule != ENUMGPU_PIVOT_RELATIVE) return fail(ENUMGPU_ERR_ARG, "unknown pivot_rule %d", r->rule);
     r->eps_feas = (o && o->eps_feas >= 0) ? o->eps_feas : 1e-9;
     r->eps_piv = (o && o->eps_piv >= 0) ? o->eps_piv : (r->rule == ENUMGPU_PIVOT_RELATIVE ? (double)p->m * 0x1p-52 : 1e-9);
+    // -0.0 passes the tests above and means 0.  Store +0.0: k_shared classifies leaf components by the high word of
+    // -eps_feas, whose sign bit must be set (with -(-0.0) = +0.0 every positive component would count as negative).
+    if (r->eps_feas == 0.0) r->eps_feas = 0.0;
+    if (r->eps_piv == 0.0) r->eps_piv = 0.0;
     r->begin = o ? o->rank_begin : 0;
     r->end = o ? o->rank_end : 0;
     if (r->begin == 0 && r->end == 0) r->end = r->total;
