@@ -73,6 +73,28 @@ class Partial(C.Structure):
 
 assert C.sizeof(Partial) == 256, C.sizeof(Partial)
 
+BASIS_FEASIBLE = 0
+BASIS_INFEASIBLE = 1
+BASIS_SINGULAR = 2
+
+CERT_OPTIMAL = 0
+CERT_BOUNDED = 1
+CERT_UNBOUNDED = 2
+CERT_UNDECIDED = 3
+
+
+class Certificate(C.Structure):
+    _fields_ = [
+        ("status", C.c_int32), ("basis_class", C.c_int32), ("entering", C.c_int32),
+        ("m", C.c_int32), ("n", C.c_int32), ("n_launches", C.c_int32),
+        ("objective", C.c_double),
+        ("y", C.c_double * MAX_M),
+        ("reduced_cost", C.c_double * MAX_N),
+        ("x_B", C.c_double * MAX_M),
+        ("ray", C.c_double * MAX_N),
+        ("n_aux_bases", C.c_uint64), ("n_rays", C.c_uint64),
+    ]
+
 # every symbol include/enumgpu.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "enumgpu_version": (C.c_int, []),
@@ -107,6 +129,9 @@ SYMBOLS = {
     "enumgpu_enqueue_host_h": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.POINTER(Options), C.c_void_p, C.POINTER(C.c_int32)]),
     "enumgpu_merge_records": (None, [C.c_void_p, C.c_int32, C.POINTER(Result)]),
     "enumgpu_selftest_rcp": (C.c_int, [C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_double)]),
+    "enumgpu_find_ray": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result)]),
+    "enumgpu_certify": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(C.c_int32), C.c_double,
+                                   C.POINTER(Certificate)]),
 }
 
 

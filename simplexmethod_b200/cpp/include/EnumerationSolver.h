@@ -40,7 +40,8 @@ public:
     ~EnumerationSolver() { release(); }
     EnumerationSolver(const EnumerationSolver& o)
         : problem_(o.problem_), devices_(o.devices_), algo_(o.algo_), rule_(o.rule_), eps_feas_(o.eps_feas_), eps_piv_(o.eps_piv_),
-          rank_begin_(o.rank_begin_), rank_end_(o.rank_end_), res_(o.res_), solved_(o.solved_) {}      // handles are not shared
+          rank_begin_(o.rank_begin_), rank_end_(o.rank_end_), check_unbounded_(o.check_unbounded_), res_(o.res_), cert_(o.cert_),
+          solved_(o.solved_), certified_(o.certified_) {}      // handles are not shared
     EnumerationSolver& operator=(const EnumerationSolver&) = delete;
 
     // optional knobs (not in the reference)
@@ -49,30 +50,30 @@ public:
     void setAlgorithm(int enumgpu_algo) { algo_ = enumgpu_algo; }
     void setTolerances(double eps_feas, double eps_piv) { eps_feas_ = eps_feas; eps_piv_ = eps_piv; }
     void setRankRange(uint64_t begin, uint64_t end) { rank_begin_ = begin; rank_end_ = end; }
+    // solve() then certifies its optimum and throws std::runtime_error("objective is unbounded") on an unbounded
+    // LP, as the reference's Solver does (SimplexSolover.h:443); needs the whole rank range.  The entry point is
+    // held as a pointer so that a program which never turns the check on links only the entries it uses.
+    void setCheckUnbounded(bool on) { check_unbounded_ = on ? &enumgpu_certify : nullptr; }
 
     Eigen::VectorXd solve()
     {
         const Eigen::MatrixXd& A = problem_.GetConstraintsMatrix();
-        enumgpu_problem p{};
-        p.m = static_cast<int32_t>(A.rows());
-        p.n = static_cast<int32_t>(A.cols());
-        p.lda = p.m;
-        p.maximize = problem_.IsMaximization() ? 1 : 0;
-        p.A_colmajor = A.data();
-        p.b = problem_.GetRightHandSide().data();
-        p.c = problem_.GetObjectiveCoefficients().data();
-        enumgpu_options o{};
-        o.eps_feas = eps_feas_; o.eps_piv = eps_piv_;
+        const enumgpu_problem p = problemStruct();
+        enumgpu_options o = options();
         o.rank_begin = rank_begin_; o.rank_end = rank_end_;
-        o.algo = algo_;
-        o.pivot_rule = rule_;
+        o.n_devices = 0; o.devices = nullptr;                     // the handles name the devices
+        if (check_unbounded_ && (rank_begin_ | rank_end_) && !(rank_begin_ == 0 && rank_end_ == binomial(p.n, p.m)))
+            throw std::invalid_argument("EnumerationSolver: setCheckUnbounded needs the whole rank range");
         int rc = acquire();
         if (rc == ENUMGPU_OK) rc = enumgpu_solve_hv(handles_.data(), static_cast<int32_t>(handles_.size()), &p, &o, &res_);
         else res_.status = rc;
         solved_ = true;
+        certified_ = false;
         if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
         if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
         if (rc == ENUMGPU_NO_FEASIBLE) throw std::runtime_error("the problem has no feasible basic solution");
+        if (check_unbounded_ && certifyWith(check_unbounded_, -1.0).status == ENUMGPU_CERT_UNBOUNDED)
+            throw std::runtime_error("objective is unbounded");
         Eigen::VectorXd x = Eigen::VectorXd::Zero(A.cols());
         for (int i = 0; i < res_.m; ++i) x[res_.basis[i]] = res_.x_B[i];
         const int n_orig = problem_.GetOriginalVariablesCount();
@@ -91,8 +92,59 @@ public:
     uint64_t feasibleCount() const { need(); return res_.n_feasible; }
     double   kernelMilliseconds() const { need(); return res_.kernel_ms; }
 
+    // Certificate of the optimal basis of the last solve() (enumgpu_certify): dual values y, reduced costs, and the
+    // verdict ENUMGPU_CERT_OPTIMAL / _BOUNDED / _UNBOUNDED (with a ray) / _UNDECIDED.  eps_opt < 0: 1e-9.
+    const enumgpu_certificate& certify(double eps_opt = -1.0) { return certifyWith(&enumgpu_certify, eps_opt); }
+    const enumgpu_certificate& certificate() const
+    {
+        if (!certified_) throw std::logic_error("EnumerationSolver: certify() has not been called");
+        return cert_;
+    }
+
 private:
     void need() const { if (!solved_) throw std::logic_error("EnumerationSolver: solve() has not been called"); }
+    using CertifyFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const int32_t*, double, enumgpu_certificate*);
+    const enumgpu_certificate& certifyWith(CertifyFn fn, double eps_opt)
+    {
+        need();
+        if (res_.status != ENUMGPU_OK) throw std::runtime_error("the problem has no feasible basic solution");
+        const enumgpu_problem p = problemStruct();
+        const enumgpu_options o = options();
+        const int rc = fn(&p, &o, res_.basis, eps_opt, &cert_);
+        if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
+        if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
+        certified_ = true;
+        return cert_;
+    }
+    static uint64_t binomial(int n, int k)          // C(n, k) for n <= 64, k <= 16: exact in 64 bits
+    {
+        uint64_t r = 1;
+        for (int i = 1; i <= k; ++i) r = r * static_cast<uint64_t>(n - k + i) / static_cast<uint64_t>(i);
+        return r;
+    }
+    enumgpu_problem problemStruct() const
+    {
+        const Eigen::MatrixXd& A = problem_.GetConstraintsMatrix();
+        enumgpu_problem p{};
+        p.m = static_cast<int32_t>(A.rows());
+        p.n = static_cast<int32_t>(A.cols());
+        p.lda = p.m;
+        p.maximize = problem_.IsMaximization() ? 1 : 0;
+        p.A_colmajor = A.data();
+        p.b = problem_.GetRightHandSide().data();
+        p.c = problem_.GetObjectiveCoefficients().data();
+        return p;
+    }
+    enumgpu_options options() const
+    {
+        enumgpu_options o{};
+        o.eps_feas = eps_feas_; o.eps_piv = eps_piv_;
+        o.algo = algo_;
+        o.pivot_rule = rule_;
+        o.n_devices = static_cast<int32_t>(devices_.size());
+        o.devices = devices_.empty() ? nullptr : devices_.data();
+        return o;
+    }
     int acquire()
     {
         if (!handles_.empty()) return ENUMGPU_OK;
@@ -117,6 +169,8 @@ private:
     int algo_ = ENUMGPU_ALGO_AUTO, rule_ = ENUMGPU_PIVOT_ABSOLUTE;
     double eps_feas_ = -1.0, eps_piv_ = -1.0;
     uint64_t rank_begin_ = 0, rank_end_ = 0;
+    CertifyFn check_unbounded_ = nullptr;      // &enumgpu_certify when setCheckUnbounded(true)
     enumgpu_result res_{};
-    bool solved_ = false;
+    enumgpu_certificate cert_{};
+    bool solved_ = false, certified_ = false;
 };

@@ -168,18 +168,16 @@ __global__ void k_empty_record(int m, int algo_used, enumgpu_partial* __restrict
     *out = r;
 }
 
-// One basis of ANY size (the device side of enumgpu_eval_basis, which stands in for Canonical::GetBasicSolution /
-// IsFeasibleBasis of a Canonical of any dimensions): one block, the frozen arithmetic of DESIGN.md §3 on
-// W = [B | b] (column-major, m x (m+1), in global memory, overwritten).  Every element receives the same operations
-// in the same order as in eval_basis_generic — the block only spreads independent elements of one step over its
-// threads; the data-dependent decisions (pivot search, thresholds, objective) are made by thread 0 in index order.
-// out: x[0..m), then z, then the class as a double.
-__global__ void __launch_bounds__(256)
-k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double thr, double eps_feas,
-           int pivot_rule, double rel_eps, double* __restrict__ rinv, double* __restrict__ out)
+// Block-wide partial-pivot elimination of W = [B | further columns] (column-major, m rows, `width` >= m+1 columns,
+// in global memory, overwritten), the frozen arithmetic of DESIGN.md §3: every column right of B receives the same
+// operations in the same order as column m (= b) does in eval_basis_generic, so adding columns changes no bit of
+// the others.  The block only spreads independent elements of one step over its threads; the data-dependent
+// decisions (pivot search, thresholds) are made by thread 0 in index order.  Returns true (on every thread) if the
+// basis is singular under pivot_rule.
+__device__ bool block_eliminate(double* __restrict__ W, int m, int width, double thr, int pivot_rule, double rel_eps,
+                                double* __restrict__ rinv)
 {
     __shared__ int s_p, s_stop;
-    __shared__ double s_x;
     const int tid = threadIdx.x, nt = blockDim.x;
     const size_t ld = (size_t)m;
     double pmax = 0.0, pmin = __longlong_as_double(0x7ff0000000000000LL);   // thread 0 only
@@ -197,14 +195,14 @@ k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double 
             if (best < pmin) pmin = best;
         }
         __syncthreads();
-        if (s_stop) { if (tid == 0) out[m + 1] = 2.0; return; }
+        if (s_stop) return true;
         const int p = s_p;
         if (p != k)
-            for (int j = k + tid; j <= m; j += nt) { const double t = W[k + j * ld]; W[k + j * ld] = W[p + j * ld]; W[p + j * ld] = t; }
+            for (int j = k + tid; j < width; j += nt) { const double t = W[k + j * ld]; W[k + j * ld] = W[p + j * ld]; W[p + j * ld] = t; }
         __syncthreads();
         const double ri = __drcp_rn(W[k + k * ld]);
         if (tid == 0) rinv[k] = ri;
-        const int rows = m - 1 - k, cols = m - k;                 // rows k+1..m-1, columns k+1..m
+        const int rows = m - 1 - k, cols = width - 1 - k;         // rows k+1..m-1, columns k+1..width-1
         for (long long e = tid; e < (long long)rows * cols; e += nt) {
             const int r = k + 1 + (int)(e % rows), j = k + 1 + (int)(e / rows);
             W[r + j * ld] = fnma(__dmul_rn(W[r + k * ld], ri), W[k + j * ld], W[r + j * ld]);
@@ -213,14 +211,23 @@ k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double 
     }
     if (tid == 0) s_stop = (pivot_rule == ENUMGPU_PIVOT_RELATIVE) && !(pmin > __dmul_rn(rel_eps, pmax));
     __syncthreads();
-    if (s_stop) { if (tid == 0) out[m + 1] = 2.0; return; }
+    return s_stop;
+}
+
+// Column sweep of column m of an eliminated W: x[0..m) and, on thread 0, z and the class (0 feasible, 1 infeasible).
+__device__ void block_solve_x(double* __restrict__ W, const double* __restrict__ cB, int m, double eps_feas,
+                              const double* __restrict__ rinv, double* __restrict__ x, double* z_out, int* cls_out)
+{
+    __shared__ double s_x;
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const size_t ld = (size_t)m;
     bool infeasible = false;       // thread 0 only
     double z = 0.0;
     for (int j = m - 1; j >= 0; --j) {
         if (tid == 0) {
             const double xj = __dmul_rn(W[j + m * ld], rinv[j]);
             s_x = xj;
-            out[j] = xj;
+            x[j] = xj;
             infeasible |= !(xj >= -eps_feas);
             z = __fma_rn(cB[j], xj, z);
         }
@@ -229,7 +236,85 @@ k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double 
         for (int i = tid; i < j; i += nt) W[i + m * ld] = fnma(W[i + j * ld], xj, W[i + m * ld]);
         __syncthreads();
     }
-    if (tid == 0) { out[m] = z; out[m + 1] = infeasible ? 1.0 : 0.0; }
+    if (tid == 0) { *z_out = z; *cls_out = infeasible ? 1 : 0; }
+}
+
+// One basis of ANY size (the device side of enumgpu_eval_basis, which stands in for Canonical::GetBasicSolution /
+// IsFeasibleBasis of a Canonical of any dimensions): one block on W = [B | b] (m x (m+1)).
+// out: x[0..m), then z, then the class as a double.
+__global__ void __launch_bounds__(256)
+k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double thr, double eps_feas,
+           int pivot_rule, double rel_eps, double* __restrict__ rinv, double* __restrict__ out)
+{
+    if (block_eliminate(W, m, m + 1, thr, pivot_rule, rel_eps, rinv)) { if (threadIdx.x == 0) out[m + 1] = 2.0; return; }
+    double z;
+    int cls;
+    block_solve_x(W, cB, m, eps_feas, rinv, out, &z, &cls);
+    if (threadIdx.x == 0) { out[m] = z; out[m + 1] = (double)cls; }
+}
+
+// The certificate of one basis (enumgpu_certify, DESIGN.md §3): one block on
+// W = [B | b | A_0 .. A_{n-1} | e_0 .. e_{m-1}] (m x (2m+n+1)).  After the shared elimination and x, thread t sweeps
+// extra column t: u_j = B^-1 a_j and r_j for t = j < n, w_i = B^-1 e_i and y_i for t = n+i.  Thread 0 then decides
+// the verdict in column order.  S: the basis (positions of B's columns in A); c: all n costs.
+constexpr int kCertifyThreads = 128;
+static_assert(kCertifyThreads >= kMaxN + kMaxM, "one thread per extra column");
+__global__ void __launch_bounds__(kCertifyThreads)
+k_certify(double* __restrict__ W, const double* __restrict__ cB, const double* __restrict__ c, const int* __restrict__ S,
+          int m, int n, int maximize, double thr, double eps_feas, int pivot_rule, double rel_eps, double eps_opt,
+          double* __restrict__ rinv, enumgpu_certificate* __restrict__ out)
+{
+    const int tid = threadIdx.x;
+    const size_t ld = (size_t)m;
+    if (tid == 0) { out->m = m; out->n = n; out->entering = -1; }
+    if (block_eliminate(W, m, 2 * m + n + 1, thr, pivot_rule, rel_eps, rinv)) {
+        if (tid == 0) { out->basis_class = ENUMGPU_BASIS_SINGULAR; out->status = ENUMGPU_CERT_UNDECIDED; }
+        return;
+    }
+    int cls = 0;
+    block_solve_x(W, cB, m, eps_feas, rinv, out->x_B, &out->objective, &cls);
+    if (tid < n + m) {                      // the same column sweep as for x, on column m+1+tid
+        double* col = W + (size_t)(m + 1 + tid) * ld;
+        double t[kMaxM];
+        for (int i = 0; i < m; ++i) t[i] = col[i];
+        double acc = tid < n ? c[tid] : 0.0;
+        for (int k = m - 1; k >= 0; --k) {
+            const double uk = __dmul_rn(t[k], rinv[k]);
+            col[k] = uk;
+            for (int i = 0; i < k; ++i) t[i] = fnma(W[i + k * ld], uk, t[i]);
+        }
+        for (int k = m - 1; k >= 0; --k)
+            acc = tid < n ? fnma(cB[k], col[k], acc) : __fma_rn(cB[k], col[k], acc);
+        if (tid < n) out->reduced_cost[tid] = acc;
+        else out->y[tid - n] = acc;
+    }
+    __syncthreads();
+    if (tid != 0) return;
+    out->basis_class = cls;
+    int entering = -1;
+    bool improving = false, nan = false;
+    for (int j = 0; j < n; ++j) {
+        bool basic = false;
+        for (int k = 0; k < m; ++k) basic |= (S[k] == j);
+        if (basic) continue;
+        const double r = out->reduced_cost[j], rk = maximize ? -r : r;
+        if (rk != rk) { nan = true; continue; }
+        if (!(rk < -eps_opt)) continue;
+        improving = true;
+        if (entering >= 0) continue;
+        const double* u = W + (size_t)(m + 1 + j) * ld;
+        bool ray = true;
+        for (int k = 0; k < m; ++k) ray &= (u[k] <= eps_opt);
+        if (ray) entering = j;
+    }
+    for (int j = 0; j < n; ++j) out->ray[j] = 0.0;
+    if (entering >= 0) {
+        const double* u = W + (size_t)(m + 1 + entering) * ld;
+        for (int k = 0; k < m; ++k) out->ray[S[k]] = -u[k];
+        out->ray[entering] = 1.0;
+    }
+    out->entering = entering;
+    out->status = entering >= 0 ? ENUMGPU_CERT_UNBOUNDED : (!improving && !nan) ? ENUMGPU_CERT_OPTIMAL : ENUMGPU_CERT_UNDECIDED;
 }
 
 // Register-resident DFMA chains: the measured FP64 roofline denominator.  kChains independent chains per thread;
@@ -1461,6 +1546,138 @@ extern "C" int enumgpu_solve(const enumgpu_problem* p, const enumgpu_options* o,
     memcpy(g_err, keep, sizeof keep);
     if (rc < 0) out->status = rc;
     return rc < 0 ? rc : out->status;
+}
+
+// ------------------------------------------------------------------ certificate and rays (DESIGN.md §3)
+
+static enumgpu_options whole_space_options(const enumgpu_options* o)
+{
+    enumgpu_options oc{};
+    oc.eps_feas = oc.eps_piv = -1.0;
+    if (o) oc = *o;
+    oc.rank_begin = oc.rank_end = 0;
+    oc.shard_index = oc.shard_count = 0;
+    return oc;
+}
+
+// The auxiliary LP [A; s*ck'] d = (0, ..., 0, -1), cost 0, minimise: its feasible bases are the extreme rays of
+// {d >= 0, A d = 0} with ck.d < 0.  s = 2^e, the largest power of two with s*max|ck_j| <= max|A_ij|, keeps
+// max|A'_ij| = max|A_ij| and with it the pivot threshold.
+extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options* o, enumgpu_result* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "out is NULL");
+    memset(out, 0, sizeof *out);
+    Resolved rs;
+    const enumgpu_options oc = whole_space_options(o);   // the caller's rank range is one of the auxiliary space
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc) return out->status = rc;
+    const int m = p->m, n = p->n, ma = m + 1;
+    if (ma > kMaxM) return out->status = fail(ENUMGPU_ERR_ARG, "find_ray: the auxiliary LP needs m+1 = %d rows, above %d", ma, kMaxM);
+    double amax = 0.0, cmax = 0.0;
+    for (int j = 0; j < n; ++j) {
+        cmax = fmax(cmax, fabs(p->c[j]));
+        for (int i = 0; i < m; ++i) amax = fmax(amax, fabs(p->A_colmajor[i + (size_t)j * p->lda]));
+    }
+    out->m = ma;
+    if (n < ma || cmax == 0.0) {          // no basis of m+1 columns, or no direction can decrease ck.x
+        out->key = INFINITY; out->best_rank = UINT64_MAX; out->objective = NAN;
+        return out->status = ENUMGPU_NO_FEASIBLE;
+    }
+    if (amax == 0.0) return out->status = fail(ENUMGPU_ERR_RANGE, "find_ray: A = 0 leaves no scale for the cost row");
+    int ea = 0, ec = 0;
+    const double fa = frexp(amax, &ea), fc = frexp(cmax, &ec);
+    const int e = ea - ec - (fc > fa ? 1 : 0);
+    std::vector<double> Aa((size_t)ma * n), ba(ma, 0.0), ca(n, 0.0);
+    for (int j = 0; j < n; ++j) {
+        for (int i = 0; i < m; ++i) Aa[(size_t)j * ma + i] = p->A_colmajor[i + (size_t)j * p->lda];
+        const double ck = p->maximize ? -p->c[j] : p->c[j];
+        const double v = ldexp(ck, e);
+        if (ldexp(v, -e) != ck) return out->status = fail(ENUMGPU_ERR_RANGE, "find_ray: c[%d] * 2^%d is not exact", j, e);
+        Aa[(size_t)j * ma + m] = v;
+    }
+    ba[m] = -1.0;
+    const enumgpu_problem aux{ma, n, ma, 0, Aa.data(), ba.data(), ca.data()};
+    return enumgpu_solve(&aux, o, out);
+}
+
+extern "C" int enumgpu_certify(const enumgpu_problem* p, const enumgpu_options* o, const int32_t* basis, double eps_opt,
+                               enumgpu_certificate* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "certify: out is NULL");
+    memset(out, 0, sizeof *out);
+    out->entering = -1;
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs;
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc) return out->status = rc;
+    if (!basis) return out->status = fail(ENUMGPU_ERR_ARG, "certify: basis is NULL");
+    const int m = p->m, n = p->n, width = 2 * m + n + 1;
+    for (int i = 0; i < m; ++i)
+        if (basis[i] < 0 || basis[i] >= n) return out->status = fail(ENUMGPU_ERR_ARG, "certify: basis index %d out of range", basis[i]);
+    if (!(eps_opt >= 0)) eps_opt = 1e-9;                 // negative (or NaN): the default
+    if (eps_opt == 0.0) eps_opt = 0.0;                   // -0.0 means 0
+    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    // W = [B | b | A | I] column-major (lda = m), then c_B, c, room for 1/pivot; the basis as int32
+    const size_t w_elems = (size_t)m * width;
+    std::vector<double> stage(w_elems + 2 * (size_t)m + n, 0.0);
+    double scale = 0.0;
+    for (int j = 0; j < n; ++j)
+        for (int i = 0; i < m; ++i) {
+            const double v = p->A_colmajor[i + (size_t)j * p->lda];
+            stage[(size_t)(m + 1 + j) * m + i] = v;
+            scale = fmax(scale, fabs(v));
+        }
+    for (int j = 0; j < m; ++j) memcpy(&stage[(size_t)j * m], p->A_colmajor + (size_t)basis[j] * p->lda, sizeof(double) * m);
+    memcpy(&stage[(size_t)m * m], p->b, sizeof(double) * m);
+    for (int i = 0; i < m; ++i) stage[(size_t)(m + 1 + n + i) * m + i] = 1.0;
+    for (int j = 0; j < m; ++j) stage[w_elems + j] = p->c[basis[j]];
+    memcpy(&stage[w_elems + m], p->c, sizeof(double) * n);
+    const double thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * scale;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    keep_pool_memory(dev);
+    cudaStream_t st = nullptr;
+    CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    auto body = [&]() -> int {
+        StreamBuf b_in, b_S, b_out;
+        CU(b_in.alloc(stage.size() * sizeof(double), st));
+        CU(b_S.alloc(sizeof(int32_t) * m, st));
+        CU(b_out.alloc(sizeof(enumgpu_certificate), st));
+        double* d_in = b_in.as<double>();
+        CU(cudaMemcpyAsync(d_in, stage.data(), stage.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(b_S.p, basis, sizeof(int32_t) * m, cudaMemcpyHostToDevice, st));
+        CU(cudaMemsetAsync(b_out.p, 0, sizeof(enumgpu_certificate), st));
+        k_certify<<<1, kCertifyThreads, 0, st>>>(d_in, d_in + w_elems, d_in + w_elems + m, b_S.as<int>(), m, n, p->maximize ? 1 : 0,
+                                                 thr, rs.eps_feas, rs.rule, rs.eps_piv, eps_opt, d_in + w_elems + m + n,
+                                                 b_out.as<enumgpu_certificate>());
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(out, b_out.p, sizeof(enumgpu_certificate), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        return 0;
+    };
+    rc = body();
+    cudaStreamDestroy(st);
+    if (rc) { out->status = rc; return rc; }
+    out->n_launches = 1;
+    if (out->basis_class != ENUMGPU_BASIS_FEASIBLE)
+        return out->status = fail(ENUMGPU_ERR_ARG, "certify: the basis is %s", out->basis_class == ENUMGPU_BASIS_SINGULAR ? "singular" : "infeasible");
+    if (out->status != ENUMGPU_CERT_UNDECIDED || m + 1 > kMaxM) return ENUMGPU_OK;
+    // a degenerate vertex: decide by enumerating the extreme rays
+    enumgpu_result aux;
+    rc = enumgpu_find_ray(p, &oc, &aux);
+    if (rc < 0) return out->status = rc;
+    out->n_launches += aux.n_launches;
+    out->n_aux_bases = aux.n_bases;
+    out->n_rays = aux.n_feasible;
+    if (rc == ENUMGPU_OK) {
+        out->status = ENUMGPU_CERT_UNBOUNDED;
+        for (int i = 0; i < aux.m; ++i) out->ray[aux.basis[i]] = aux.x_B[i];
+    } else if (aux.n_feasible == 0) {
+        out->status = ENUMGPU_CERT_BOUNDED;
+    }                                     // feasible aux bases whose key is NaN (overflow): stays UNDECIDED
+    return ENUMGPU_OK;
 }
 
 #ifdef ENUMGPU_TRACE

@@ -165,7 +165,10 @@ class EnumerationSolver:
 
     def __init__(self, problem: Canonical, devices: Optional[Sequence[int]] = None,
                  algo: int = _abi.ALGO_AUTO, eps_feas: float = 1e-9, eps_piv: float = -1.0,
-                 pivot_rule: int = _abi.PIVOT_ABSOLUTE):
+                 pivot_rule: int = _abi.PIVOT_ABSOLUTE, check_unbounded: bool = False):
+        """check_unbounded: solve() certifies the enumeration's optimum (certify()) and raises
+        RuntimeError("objective is unbounded") on an unbounded LP, as the reference's Solver does
+        (SimplexSolover.h:443).  Off by default: enumerating vertices alone cannot see unboundedness."""
         A = problem.GetConstraintsMatrix()
         m, n = A.shape
         if m > n:
@@ -177,7 +180,9 @@ class EnumerationSolver:
         self._algo = int(algo)
         self._eps = (float(eps_feas), float(eps_piv))      # eps_piv < 0: the rule's default (1e-9 absolute, m*2^-52 relative)
         self._rule = int(pivot_rule)
+        self._check_unbounded = bool(check_unbounded)
         self._res: Optional[_abi.Result] = None
+        self._cert: Optional[_abi.Certificate] = None
         self._handles = None                         # enumgpu_handle per device, created at the first solve, kept
 
     # -- handles: stream, events, pinned staging, device buffers live as long as the solver (include/enumgpu.h) --
@@ -214,10 +219,16 @@ class EnumerationSolver:
 
     # -- the reference call shape ------------------------------------------
     def solve(self, rank_begin: int = 0, rank_end: int = 0) -> np.ndarray:
+        p = self._problem
+        if self._check_unbounded and (rank_begin, rank_end) != (0, 0):
+            m, n = p.GetConstraintsMatrix().shape
+            if (rank_begin, rank_end) != (0, lib().enumgpu_binomial(n, m)):
+                raise ValueError("check_unbounded needs the whole rank range: its conclusion rests on the global optimum")
         res = self.enumerate(rank_begin, rank_end)
         if res.status == _abi.NO_FEASIBLE:
             raise RuntimeError("the problem has no feasible basic solution")
-        p = self._problem
+        if self._check_unbounded and self.certify().status == _abi.CERT_UNBOUNDED:
+            raise RuntimeError("objective is unbounded")
         x = np.zeros(p.GetObjectiveCoefficients().size)
         for i in range(res.m):
             x[res.basis[i]] = res.x_B[i]
@@ -240,7 +251,58 @@ class EnumerationSolver:
         rc = lib().enumgpu_solve_hv(arr, len(hs), C.byref(ps), C.byref(o), C.byref(res))
         _check(rc)
         self._res = res
+        self._cert = None
         return res
+
+    # -- certificate of the optimum: duals, reduced costs, unboundedness (enumgpu_certify) --------
+    def _device_options(self):
+        """Options for the handle-free entries: the solver's device list, tolerances, kernel and rule."""
+        o = self._options()
+        if self._devices:
+            self._dev_arr = (C.c_int32 * len(self._devices))(*self._devices)
+            o.n_devices, o.devices = len(self._devices), self._dev_arr
+        return o
+
+    def certify(self, eps_opt: float = 1e-9) -> _abi.Certificate:
+        """Certificate of the last enumeration's optimal basis (enumerates first if nothing has been).
+        .status is CERT_OPTIMAL (y dual feasible), CERT_BOUNDED (degenerate vertex: no ray exists, y not dual
+        feasible), CERT_UNBOUNDED (.ray is a ray) or CERT_UNDECIDED (degenerate vertex at m = 16)."""
+        res = self._res if self._res is not None else self.enumerate()
+        if res.status != _abi.OK:
+            raise RuntimeError("the problem has no feasible basic solution")
+        p = self._problem
+        ps = _problem_struct(p.GetConstraintsMatrix(), p.GetRightHandSide(), p.GetObjectiveCoefficients(), p.IsMaximization())
+        basis = (C.c_int32 * res.m)(*list(res.basis)[:res.m])
+        cert = _abi.Certificate()
+        _check(lib().enumgpu_certify(C.byref(ps), C.byref(self._device_options()), basis, float(eps_opt), C.byref(cert)))
+        self._cert = cert
+        return cert
+
+    def findRay(self) -> _abi.Result:
+        """enumgpu_find_ray: the extreme rays of {d >= 0, A d = 0} with c.d < 0 (> 0 when maximising), enumerated as
+        the feasible bases of the auxiliary LP of include/enumgpu.h.  status OK: basis/x_B of the lowest-rank ray."""
+        p = self._problem
+        ps = _problem_struct(p.GetConstraintsMatrix(), p.GetRightHandSide(), p.GetObjectiveCoefficients(), p.IsMaximization())
+        res = _abi.Result()
+        _check(lib().enumgpu_find_ray(C.byref(ps), C.byref(self._device_options()), C.byref(res)))
+        return res
+
+    def _need_cert(self) -> _abi.Certificate:
+        return self._cert if self._cert is not None else self.certify()
+
+    def dualValues(self) -> np.ndarray:
+        """y = B^-T c_B at the optimal basis (shadow prices, true sense)."""
+        c = self._need_cert(); return np.array(c.y[: c.m])
+
+    def reducedCosts(self) -> np.ndarray:
+        """r_j = c_j - y.a_j for every column (true sense; ~0 on the basic ones)."""
+        c = self._need_cert(); return np.array(c.reduced_cost[: c.n])
+
+    def unboundedRay(self) -> Optional[np.ndarray]:
+        """A ray d >= 0, A d = 0 along which the objective improves without bound, or None if the LP is bounded
+        (or, at m = 16 on a degenerate vertex, undecided)."""
+        c = self._need_cert()
+        return np.array(c.ray[: c.n]) if c.status == _abi.CERT_UNBOUNDED else None
 
     # -- the extreme points themselves (README step 9 of the reference) -------
     def listFeasibleBases(self, capacity: int = 1 << 22):
