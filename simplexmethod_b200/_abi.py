@@ -95,6 +95,21 @@ class Certificate(C.Structure):
         ("n_aux_bases", C.c_uint64), ("n_rays", C.c_uint64),
     ]
 
+OPT_WINNER = 0
+OPT_WINDOW = 1
+OPT_FALLBACK = 2
+
+
+class Optimum(C.Structure):
+    _fields_ = [
+        ("cert", Certificate),
+        ("basis", C.c_int32 * MAX_M),
+        ("source", C.c_int32), ("n_launches", C.c_int32),
+        ("rank", C.c_uint64), ("key_bound", C.c_double),
+        ("n_window", C.c_uint64), ("window_index", C.c_uint64),
+    ]
+
+
 # every symbol include/enumgpu.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "enumgpu_version": (C.c_int, []),
@@ -132,6 +147,12 @@ SYMBOLS = {
     "enumgpu_find_ray": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result)]),
     "enumgpu_certify": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(C.c_int32), C.c_double,
                                    C.POINTER(Certificate)]),
+    "enumgpu_list_window": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.c_double, C.POINTER(C.c_uint64),
+                                       C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(Result)]),
+    "enumgpu_certify_bases": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(C.c_int32), C.c_uint64,
+                                         C.c_double, C.POINTER(Certificate)]),
+    "enumgpu_certify_optimum": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result), C.c_double,
+                                           C.c_uint64, C.POINTER(Optimum)]),
 }
 
 

@@ -40,8 +40,8 @@ public:
     ~EnumerationSolver() { release(); }
     EnumerationSolver(const EnumerationSolver& o)
         : problem_(o.problem_), devices_(o.devices_), algo_(o.algo_), rule_(o.rule_), eps_feas_(o.eps_feas_), eps_piv_(o.eps_piv_),
-          rank_begin_(o.rank_begin_), rank_end_(o.rank_end_), check_unbounded_(o.check_unbounded_), res_(o.res_), cert_(o.cert_),
-          solved_(o.solved_), certified_(o.certified_) {}      // handles are not shared
+          rank_begin_(o.rank_begin_), rank_end_(o.rank_end_), check_unbounded_(o.check_unbounded_), optimal_duals_(o.optimal_duals_),
+          res_(o.res_), cert_(o.cert_), cert_basis_(o.cert_basis_), solved_(o.solved_), certified_(o.certified_) {}   // handles are not shared
     EnumerationSolver& operator=(const EnumerationSolver&) = delete;
 
     // optional knobs (not in the reference)
@@ -54,6 +54,11 @@ public:
     // LP, as the reference's Solver does (SimplexSolover.h:443); needs the whole rank range.  The entry point is
     // held as a pointer so that a program which never turns the check on links only the entries it uses.
     void setCheckUnbounded(bool on) { check_unbounded_ = on ? &enumgpu_certify : nullptr; }
+    // certify() (and the unboundedness check) searches all optimal bases for a dual-feasible one when the winner's
+    // certificate is undecided (enumgpu_certify_optimum); certificateBasis() then names the basis the certificate
+    // belongs to, which may differ from optimalBasis().  Off by default: it costs one more enumeration on a
+    // degenerate optimum.  Held as a pointer for the same reason as above.
+    void setOptimalDuals(bool on) { optimal_duals_ = on ? &enumgpu_certify_optimum : nullptr; }
 
     Eigen::VectorXd solve()
     {
@@ -100,6 +105,10 @@ public:
         if (!certified_) throw std::logic_error("EnumerationSolver: certify() has not been called");
         return cert_;
     }
+    // the columns (ascending) of the basis the certificate belongs to; with setOptimalDuals(true) also the window
+    // search's source (ENUMGPU_OPT_*), else ENUMGPU_OPT_WINNER
+    const std::vector<int>& certificateBasis() const { certificate(); return cert_basis_; }
+    int certificateSource() const { certificate(); return cert_source_; }
 
 private:
     void need() const { if (!solved_) throw std::logic_error("EnumerationSolver: solve() has not been called"); }
@@ -110,7 +119,18 @@ private:
         if (res_.status != ENUMGPU_OK) throw std::runtime_error("the problem has no feasible basic solution");
         const enumgpu_problem p = problemStruct();
         const enumgpu_options o = options();
-        const int rc = fn(&p, &o, res_.basis, eps_opt, &cert_);
+        int rc;
+        if (optimal_duals_) {
+            enumgpu_optimum opt{};
+            rc = optimal_duals_(&p, &o, &res_, eps_opt, 0, &opt);
+            cert_ = opt.cert;
+            cert_basis_.assign(opt.basis, opt.basis + res_.m);
+            cert_source_ = opt.source;
+        } else {
+            rc = fn(&p, &o, res_.basis, eps_opt, &cert_);
+            cert_basis_.assign(res_.basis, res_.basis + res_.m);
+            cert_source_ = ENUMGPU_OPT_WINNER;
+        }
         if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
         if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
         certified_ = true;
@@ -170,7 +190,12 @@ private:
     double eps_feas_ = -1.0, eps_piv_ = -1.0;
     uint64_t rank_begin_ = 0, rank_end_ = 0;
     CertifyFn check_unbounded_ = nullptr;      // &enumgpu_certify when setCheckUnbounded(true)
+    using OptimumFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const enumgpu_result*, double, uint64_t,
+                              enumgpu_optimum*);
+    OptimumFn optimal_duals_ = nullptr;        // &enumgpu_certify_optimum when setOptimalDuals(true)
     enumgpu_result res_{};
     enumgpu_certificate cert_{};
+    std::vector<int> cert_basis_;
+    int cert_source_ = ENUMGPU_OPT_WINNER;
     bool solved_ = false, certified_ = false;
 };

@@ -46,11 +46,13 @@ struct LaunchParams {
     uint32_t chunk;         // ranks per thread (independent kernel)
     uint32_t shard_index;   // interleaved sharding: this launch owns the work
     uint32_t shard_count;   // windows whose index is shard_index mod shard_count
-    // optional listing of the feasible bases (enumgpu_list_feasible): ranks are appended in
-    // arbitrary order; *list_count counts all of them, only the first list_cap are stored
+    // optional listing of the feasible bases (enumgpu_list_window): ranks are appended in
+    // arbitrary order; *list_count counts all of them, only the first list_cap are stored.
+    // A feasible basis is listed iff in_window(key, list_key_max) (+inf lists all of them).
     unsigned long long* list_count;
     uint64_t* list_ranks;
     uint64_t  list_cap;
+    double    list_key_max;
     // singularity rule: ENUMGPU_PIVOT_ABSOLUTE (thr above) or ENUMGPU_PIVOT_RELATIVE (thr = 0, rel_eps below;
     // the run-time-m kernels only)
     int32_t  pivot_rule;
@@ -63,6 +65,12 @@ struct LaunchParams {
     uint32_t         total_blocks;
     enumgpu_partial* record;
 };
+
+// +inf lists every feasible basis, NaN keys included; a finite bound never lists a NaN key
+__device__ __forceinline__ bool in_window(double key, double key_max)
+{
+    return key <= key_max || key_max == __longlong_as_double(0x7ff0000000000000LL);
+}
 
 __device__ __forceinline__ void list_append(unsigned long long* count, uint64_t* ranks, uint64_t cap, uint64_t rank)
 {

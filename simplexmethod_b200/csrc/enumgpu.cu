@@ -253,17 +253,31 @@ k_eval_any(double* __restrict__ W, const double* __restrict__ cB, int m, double 
     if (threadIdx.x == 0) { out[m] = z; out[m + 1] = (double)cls; }
 }
 
-// The certificate of one basis (enumgpu_certify, DESIGN.md §3): one block on
-// W = [B | b | A_0 .. A_{n-1} | e_0 .. e_{m-1}] (m x (2m+n+1)).  After the shared elimination and x, thread t sweeps
-// extra column t: u_j = B^-1 a_j and r_j for t = j < n, w_i = B^-1 e_i and y_i for t = n+i.  Thread 0 then decides
-// the verdict in column order.  S: the basis (positions of B's columns in A); c: all n costs.
+// The certificate of a basis (enumgpu_certify, DESIGN.md §3): block i certifies basis S_all[i*m .. i*m+m) in its own
+// slab of scratch (certify_slab doubles): W = [B | b | A_0 .. A_{n-1} | e_0 .. e_{m-1}] (m x (2m+n+1)), then c_B and
+// room for 1/pivot; it writes out_all[i].  After the shared elimination and x, thread t sweeps extra column t:
+// u_j = B^-1 a_j and r_j for t = j < n, w_i = B^-1 e_i and y_i for t = n+i.  Thread 0 then decides the verdict in
+// column order.  A: packed (lda = m); c: all n costs.
 constexpr int kCertifyThreads = 128;
 static_assert(kCertifyThreads >= kMaxN + kMaxM, "one thread per extra column");
+__host__ __device__ inline size_t certify_slab(int m, int n) { return (size_t)m * (2 * m + n + 1) + 2 * (size_t)m; }
 __global__ void __launch_bounds__(kCertifyThreads)
-k_certify(double* __restrict__ W, const double* __restrict__ cB, const double* __restrict__ c, const int* __restrict__ S,
-          int m, int n, int maximize, double thr, double eps_feas, int pivot_rule, double rel_eps, double eps_opt,
-          double* __restrict__ rinv, enumgpu_certificate* __restrict__ out)
+k_certify(const double* __restrict__ A, const double* __restrict__ b, const double* __restrict__ c,
+          const int* __restrict__ S_all, int m, int n, int maximize, double thr, double eps_feas, int pivot_rule,
+          double rel_eps, double eps_opt, double* __restrict__ scratch, enumgpu_certificate* __restrict__ out_all)
 {
+    const int* __restrict__ S = S_all + (size_t)blockIdx.x * m;
+    double* __restrict__ W = scratch + (size_t)blockIdx.x * certify_slab(m, n);
+    double* __restrict__ cB = W + (size_t)m * (2 * m + n + 1);
+    double* __restrict__ rinv = cB + m;
+    enumgpu_certificate* __restrict__ out = out_all + blockIdx.x;
+    for (int e = threadIdx.x; e < m * (2 * m + n + 1); e += blockDim.x) {
+        const int j = e / m, r = e - j * m;
+        W[e] = j < m ? A[r + (size_t)S[j] * m] : j == m ? b[r] : j <= m + n ? A[r + (size_t)(j - m - 1) * m]
+             : (r == j - m - 1 - n ? 1.0 : 0.0);
+    }
+    for (int j = threadIdx.x; j < m; j += blockDim.x) cB[j] = c[S[j]];
+    __syncthreads();
     const int tid = threadIdx.x;
     const size_t ld = (size_t)m;
     if (tid == 0) { out->m = m; out->n = n; out->entering = -1; }
@@ -638,7 +652,8 @@ static bool shared_rcp_trusted(int dev);
 static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Resolved& rs, uint64_t begin, uint64_t end,
                          uint32_t shard_index, uint32_t shard_count,
                          cudaStream_t st, enumgpu_partial* partial_dev, int32_t* n_launches, Scratch* scratch = nullptr,
-                         unsigned long long* list_count = nullptr, uint64_t* list_ranks = nullptr, uint64_t list_cap = 0)
+                         unsigned long long* list_count = nullptr, uint64_t* list_ranks = nullptr, uint64_t list_cap = 0,
+                         double list_key_max = INFINITY)
 {
     int launches = 0;
     int dev = 0, sms = 148;
@@ -672,7 +687,7 @@ static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Res
     prm.rel_eps = rs.rule == ENUMGPU_PIVOT_RELATIVE ? rs.eps_piv : 0.0;
     prm.rank_begin = begin; prm.rank_end = end; prm.chunk = 1;
     prm.shard_index = 0; prm.shard_count = 1;
-    prm.list_count = list_count; prm.list_ranks = list_ranks; prm.list_cap = list_cap;
+    prm.list_count = list_count; prm.list_ranks = list_ranks; prm.list_cap = list_cap; prm.list_key_max = list_key_max;
     const bool first_shard = (shard_index == 0), last_shard = (shard_index + 1 == shard_count);
 
     int algo = rs.algo;
@@ -1029,14 +1044,16 @@ static int upload_problem(const enumgpu_problem* p, cudaStream_t st, DeviceProbl
     return 0;
 }
 
-extern "C" int enumgpu_list_feasible(const enumgpu_problem* p, const enumgpu_options* o, uint64_t* ranks, uint64_t capacity,
-                                     uint64_t* n_listed, enumgpu_result* out)
+// enumgpu_list_window into `ranks` (capacity entries), or, with `fit`, into *fit resized to the number listed (the
+// library's own callers, which ask for a large capacity and usually receive a few entries).
+static int list_window(const enumgpu_problem* p, const enumgpu_options* o, double key_max, uint64_t* ranks, uint64_t capacity,
+                       std::vector<uint64_t>* fit, uint64_t* n_listed, enumgpu_result* out, uint64_t* n_window = nullptr)
 {
     g_err[0] = 0;
-    if (!out || !n_listed) return fail(ENUMGPU_ERR_ARG, "list_feasible: NULL argument");
+    if (!out || !n_listed) return fail(ENUMGPU_ERR_ARG, "list_window: NULL argument");
     memset(out, 0, sizeof *out);
     *n_listed = 0;
-    if (capacity && !ranks) return out->status = fail(ENUMGPU_ERR_ARG, "list_feasible: ranks is NULL but capacity is %llu", (unsigned long long)capacity);
+    if (capacity && !ranks && !fit) return out->status = fail(ENUMGPU_ERR_ARG, "list_window: ranks is NULL but capacity is %llu", (unsigned long long)capacity);
     Resolved rs;
     int rc = resolve(p, o, &rs, true);
     if (rc) return out->status = rc;
@@ -1064,13 +1081,15 @@ extern "C" int enumgpu_list_feasible(const enumgpu_problem* p, const enumgpu_opt
         CU(cudaEventCreate(&e1));
         CU(cudaEventRecord(e0, st));
         r2 = enqueue_range(&D.dp, D.scale, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, b_part.as<enumgpu_partial>(),
-                           &launches, nullptr, b_count.as<unsigned long long>(), b_ranks.as<uint64_t>(), capacity);
+                           &launches, nullptr, b_count.as<unsigned long long>(), b_ranks.as<uint64_t>(), capacity, key_max);
         if (r2) return r2;
         CU(cudaEventRecord(e1, st));
         CU(cudaMemcpyAsync(&h_part, b_part.p, sizeof h_part, cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(&h_count, b_count.p, sizeof h_count, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         const uint64_t k = h_count < capacity ? (uint64_t)h_count : capacity;
+        if (fit) { fit->resize(k); ranks = fit->data(); }
+        if (n_window) *n_window = h_count;
         if (k) CU(cudaMemcpy(ranks, b_ranks.p, sizeof(uint64_t) * k, cudaMemcpyDeviceToHost));
         *n_listed = k;
         float ms = 0.f;
@@ -1087,6 +1106,18 @@ extern "C" int enumgpu_list_feasible(const enumgpu_problem* p, const enumgpu_opt
     if (rc) return out->status = rc;
     std::sort(ranks, ranks + *n_listed);     // the device appends in arrival order; hand them out ascending
     return out->status;
+}
+
+extern "C" int enumgpu_list_window(const enumgpu_problem* p, const enumgpu_options* o, double key_max, uint64_t* ranks,
+                                   uint64_t capacity, uint64_t* n_listed, enumgpu_result* out)
+{
+    return list_window(p, o, key_max, ranks, capacity, nullptr, n_listed, out);
+}
+
+extern "C" int enumgpu_list_feasible(const enumgpu_problem* p, const enumgpu_options* o, uint64_t* ranks, uint64_t capacity,
+                                     uint64_t* n_listed, enumgpu_result* out)
+{
+    return list_window(p, o, INFINITY, ranks, capacity, nullptr, n_listed, out);
 }
 
 extern "C" int enumgpu_eval_ranks(const enumgpu_problem* p, const enumgpu_options* o, const uint64_t* ranks, uint64_t count,
@@ -1601,72 +1632,88 @@ extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options*
     return enumgpu_solve(&aux, o, out);
 }
 
-extern "C" int enumgpu_certify(const enumgpu_problem* p, const enumgpu_options* o, const int32_t* basis, double eps_opt,
-                               enumgpu_certificate* out)
-{
-    g_err[0] = 0;
-    if (!out) return fail(ENUMGPU_ERR_ARG, "certify: out is NULL");
-    memset(out, 0, sizeof *out);
-    out->entering = -1;
-    const enumgpu_options oc = whole_space_options(o);
-    Resolved rs;
-    int rc = resolve(p, &oc, &rs, true);
-    if (rc) return out->status = rc;
-    if (!basis) return out->status = fail(ENUMGPU_ERR_ARG, "certify: basis is NULL");
-    const int m = p->m, n = p->n, width = 2 * m + n + 1;
-    for (int i = 0; i < m; ++i)
-        if (basis[i] < 0 || basis[i] >= n) return out->status = fail(ENUMGPU_ERR_ARG, "certify: basis index %d out of range", basis[i]);
-    if (!(eps_opt >= 0)) eps_opt = 1e-9;                 // negative (or NaN): the default
-    if (eps_opt == 0.0) eps_opt = 0.0;                   // -0.0 means 0
-    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
-    // W = [B | b | A | I] column-major (lda = m), then c_B, c, room for 1/pivot; the basis as int32
-    const size_t w_elems = (size_t)m * width;
-    std::vector<double> stage(w_elems + 2 * (size_t)m + n, 0.0);
-    double scale = 0.0;
-    for (int j = 0; j < n; ++j)
-        for (int i = 0; i < m; ++i) {
-            const double v = p->A_colmajor[i + (size_t)j * p->lda];
-            stage[(size_t)(m + 1 + j) * m + i] = v;
-            scale = fmax(scale, fabs(v));
-        }
-    for (int j = 0; j < m; ++j) memcpy(&stage[(size_t)j * m], p->A_colmajor + (size_t)basis[j] * p->lda, sizeof(double) * m);
-    memcpy(&stage[(size_t)m * m], p->b, sizeof(double) * m);
-    for (int i = 0; i < m; ++i) stage[(size_t)(m + 1 + n + i) * m + i] = 1.0;
-    for (int j = 0; j < m; ++j) stage[w_elems + j] = p->c[basis[j]];
-    memcpy(&stage[w_elems + m], p->c, sizeof(double) * n);
-    const double thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * scale;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    keep_pool_memory(dev);
+// k_certify on a list of bases, kCertifyChunk blocks per launch at most: the device copy of the LP, the scratch
+// slabs and the staging of the bases and certificates are sized by the chunk, not by the number of bases.
+constexpr uint32_t kCertifyChunk = 4096;
+struct Certifier {
+    struct OwnedStream {               // declared first: destroyed after the buffers have queued their frees on it
+        cudaStream_t s = nullptr;
+        ~OwnedStream() { if (s) cudaStreamDestroy(s); }
+    } owned;
     cudaStream_t st = nullptr;
-    CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    auto body = [&]() -> int {
-        StreamBuf b_in, b_S, b_out;
-        CU(b_in.alloc(stage.size() * sizeof(double), st));
-        CU(b_S.alloc(sizeof(int32_t) * m, st));
-        CU(b_out.alloc(sizeof(enumgpu_certificate), st));
-        double* d_in = b_in.as<double>();
-        CU(cudaMemcpyAsync(d_in, stage.data(), stage.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(b_S.p, basis, sizeof(int32_t) * m, cudaMemcpyHostToDevice, st));
-        CU(cudaMemsetAsync(b_out.p, 0, sizeof(enumgpu_certificate), st));
-        k_certify<<<1, kCertifyThreads, 0, st>>>(d_in, d_in + w_elems, d_in + w_elems + m, b_S.as<int>(), m, n, p->maximize ? 1 : 0,
-                                                 thr, rs.eps_feas, rs.rule, rs.eps_piv, eps_opt, d_in + w_elems + m + n,
-                                                 b_out.as<enumgpu_certificate>());
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(out, b_out.p, sizeof(enumgpu_certificate), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+    DeviceProblem D;
+    StreamBuf b_scratch, b_S, b_out;
+    double thr = 0.0;
+    int32_t launches = 0;
+
+    int init(const enumgpu_problem* p, const Resolved& rs)
+    {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        keep_pool_memory(dev);
+        CU(cudaStreamCreateWithFlags(&owned.s, cudaStreamNonBlocking));
+        st = owned.s;
+        const int rc = upload_problem(p, st, &D);
+        if (rc) return rc;
+        thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * D.scale;
+        CU(b_scratch.alloc(sizeof(double) * certify_slab(p->m, p->n) * kCertifyChunk, st));
+        CU(b_S.alloc(sizeof(int32_t) * p->m * kCertifyChunk, st));
+        CU(b_out.alloc(sizeof(enumgpu_certificate) * kCertifyChunk, st));
         return 0;
-    };
-    rc = body();
-    cudaStreamDestroy(st);
+    }
+    // count <= kCertifyChunk bases of m columns each (host); out[i] as the kernel leaves it, n_launches = 1
+    int run(const enumgpu_problem* p, const Resolved& rs, const int32_t* bases, uint32_t count, double eps_opt,
+            enumgpu_certificate* out)
+    {
+        const int m = p->m, n = p->n;
+        CU(cudaMemcpyAsync(b_S.p, bases, sizeof(int32_t) * m * count, cudaMemcpyHostToDevice, st));
+        CU(cudaMemsetAsync(b_out.p, 0, sizeof(enumgpu_certificate) * count, st));
+        k_certify<<<count, kCertifyThreads, 0, st>>>(D.dp.A_colmajor, D.dp.b, D.dp.c, b_S.as<int>(), m, n, p->maximize ? 1 : 0,
+                                                     thr, rs.eps_feas, rs.rule, rs.eps_piv, eps_opt, b_scratch.as<double>(),
+                                                     b_out.as<enumgpu_certificate>());
+        CU(cudaGetLastError());
+        ++launches;
+        CU(cudaMemcpyAsync(out, b_out.p, sizeof(enumgpu_certificate) * count, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        for (uint32_t i = 0; i < count; ++i) out[i].n_launches = 1;
+        return 0;
+    }
+};
+
+static double resolve_eps_opt(double eps_opt)
+{
+    if (!(eps_opt >= 0)) return 1e-9;                    // negative (or NaN): the default
+    return eps_opt == 0.0 ? 0.0 : eps_opt;               // -0.0 means 0
+}
+
+static int check_bases(const enumgpu_problem* p, const int32_t* bases, uint64_t count, const char* who)
+{
+    if (!bases) return fail(ENUMGPU_ERR_ARG, "%s: basis is NULL", who);
+    for (uint64_t i = 0; i < count * (uint64_t)p->m; ++i)
+        if (bases[i] < 0 || bases[i] >= p->n) return fail(ENUMGPU_ERR_ARG, "%s: basis index %d out of range", who, bases[i]);
+    return 0;
+}
+
+// The certificate of one basis without the ray fallback; ENUMGPU_ERR_ARG for a singular or infeasible basis.
+static int certify_one(const enumgpu_problem* p, const Resolved& rs, const int32_t* basis, double eps_opt,
+                       enumgpu_certificate* out)
+{
+    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    Certifier cf;
+    int rc = cf.init(p, rs);
+    if (rc == 0) rc = cf.run(p, rs, basis, 1, eps_opt, out);
     if (rc) { out->status = rc; return rc; }
-    out->n_launches = 1;
     if (out->basis_class != ENUMGPU_BASIS_FEASIBLE)
         return out->status = fail(ENUMGPU_ERR_ARG, "certify: the basis is %s", out->basis_class == ENUMGPU_BASIS_SINGULAR ? "singular" : "infeasible");
-    if (out->status != ENUMGPU_CERT_UNDECIDED || m + 1 > kMaxM) return ENUMGPU_OK;
-    // a degenerate vertex: decide by enumerating the extreme rays
+    return ENUMGPU_OK;
+}
+
+// An undecided certificate (a degenerate vertex) decided by enumerating the extreme rays, where m+1 rows fit.
+static int ray_fallback(const enumgpu_problem* p, const enumgpu_options* oc, enumgpu_certificate* out)
+{
+    if (out->status != ENUMGPU_CERT_UNDECIDED || p->m + 1 > kMaxM) return ENUMGPU_OK;
     enumgpu_result aux;
-    rc = enumgpu_find_ray(p, &oc, &aux);
+    const int rc = enumgpu_find_ray(p, oc, &aux);
     if (rc < 0) return out->status = rc;
     out->n_launches += aux.n_launches;
     out->n_aux_bases = aux.n_bases;
@@ -1678,6 +1725,111 @@ extern "C" int enumgpu_certify(const enumgpu_problem* p, const enumgpu_options* 
         out->status = ENUMGPU_CERT_BOUNDED;
     }                                     // feasible aux bases whose key is NaN (overflow): stays UNDECIDED
     return ENUMGPU_OK;
+}
+
+extern "C" int enumgpu_certify(const enumgpu_problem* p, const enumgpu_options* o, const int32_t* basis, double eps_opt,
+                               enumgpu_certificate* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "certify: out is NULL");
+    memset(out, 0, sizeof *out);
+    out->entering = -1;
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs;
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc || (rc = check_bases(p, basis, 1, "certify"))) return out->status = rc;
+    rc = certify_one(p, rs, basis, resolve_eps_opt(eps_opt), out);
+    if (rc) return rc;
+    return ray_fallback(p, &oc, out);
+}
+
+extern "C" int enumgpu_certify_bases(const enumgpu_problem* p, const enumgpu_options* o, const int32_t* bases, uint64_t count,
+                                     double eps_opt, enumgpu_certificate* out)
+{
+    g_err[0] = 0;
+    if (count && !out) return fail(ENUMGPU_ERR_ARG, "certify_bases: out is NULL");
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs;
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc || (rc = check_bases(p, bases, count, "certify_bases"))) return rc;
+    if (count == 0) return ENUMGPU_OK;
+    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    eps_opt = resolve_eps_opt(eps_opt);
+    Certifier cf;
+    if ((rc = cf.init(p, rs))) return rc;
+    for (uint64_t i = 0; i < count; i += kCertifyChunk) {
+        const uint32_t k = (uint32_t)std::min<uint64_t>(kCertifyChunk, count - i);
+        if ((rc = cf.run(p, rs, bases + i * p->m, k, eps_opt, out + i))) return rc;
+        for (uint32_t j = 0; j < k; ++j)
+            if (out[i + j].basis_class != ENUMGPU_BASIS_FEASIBLE) out[i + j].status = ENUMGPU_ERR_ARG;
+    }
+    return ENUMGPU_OK;
+}
+
+extern "C" int enumgpu_certify_optimum(const enumgpu_problem* p, const enumgpu_options* o, const enumgpu_result* opt,
+                                       double eps_opt, uint64_t max_window, enumgpu_optimum* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "certify_optimum: out is NULL");
+    memset(out, 0, sizeof *out);
+    out->cert.entering = -1;
+    out->window_index = UINT64_MAX;
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs;
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc) return out->cert.status = rc;
+    if (!opt || opt->status != ENUMGPU_OK || opt->m != p->m)
+        return out->cert.status = fail(ENUMGPU_ERR_ARG, "certify_optimum: opt is not an optimum of this LP (status OK, m = %d)", p->m);
+    const int m = p->m, n = p->n;
+    int32_t S[kMaxM];
+    if (opt->best_rank >= rs.total || enumgpu_unrank(n, m, opt->best_rank, S) != 0 || memcmp(S, opt->basis, sizeof(int32_t) * m))
+        return out->cert.status = fail(ENUMGPU_ERR_ARG, "certify_optimum: opt->basis is not unrank(opt->best_rank)");
+    eps_opt = resolve_eps_opt(eps_opt);
+    if (max_window == 0) max_window = 1ull << 24;
+    memcpy(out->basis, S, sizeof(int32_t) * m);
+    out->rank = opt->best_rank;
+    out->key_bound = opt->key + eps_opt * fmax(1.0, fabs(opt->key));
+    out->source = ENUMGPU_OPT_WINNER;
+    // 1. the winner
+    rc = certify_one(p, rs, S, eps_opt, &out->cert);
+    out->n_launches = out->cert.n_launches;
+    if (rc || out->cert.status != ENUMGPU_CERT_UNDECIDED) return rc;
+    // 2. the window: the feasible bases whose key is at most key_bound, among them every optimal basis
+    std::vector<uint64_t> window;
+    enumgpu_result lr;
+    uint64_t n_listed = 0;
+    rc = list_window(p, &oc, out->key_bound, nullptr, max_window, &window, &n_listed, &lr, &out->n_window);
+    out->n_launches += lr.n_launches;
+    if (rc < 0) return out->cert.status = rc;
+    // 3. its bases in ascending rank, a chunk at a time, up to the first chunk with an OPTIMAL one
+    if (out->n_window <= max_window) {
+        Certifier cf;
+        if ((rc = cf.init(p, rs))) return out->cert.status = rc;
+        std::vector<int32_t> bases((size_t)kCertifyChunk * m);
+        std::vector<enumgpu_certificate> certs(kCertifyChunk);
+        for (uint64_t i = 0; i < n_listed; i += kCertifyChunk) {
+            const uint32_t k = (uint32_t)std::min<uint64_t>(kCertifyChunk, n_listed - i);
+            for (uint32_t j = 0; j < k; ++j) enumgpu_unrank(n, m, window[i + j], &bases[(size_t)j * m]);
+            rc = cf.run(p, rs, bases.data(), k, eps_opt, certs.data());
+            out->n_launches += 1;
+            if (rc) return out->cert.status = rc;
+            for (uint32_t j = 0; j < k; ++j)
+                if (certs[j].basis_class == ENUMGPU_BASIS_FEASIBLE && certs[j].status == ENUMGPU_CERT_OPTIMAL) {
+                    out->cert = certs[j];
+                    memcpy(out->basis, &bases[(size_t)j * m], sizeof(int32_t) * m);
+                    out->rank = window[i + j];
+                    out->window_index = i + j;
+                    out->source = ENUMGPU_OPT_WINDOW;
+                    return ENUMGPU_OK;
+                }
+        }
+    }
+    // 4. no optimal basis in the window, or a window above max_window: enumgpu_certify's answer at the winner
+    out->source = ENUMGPU_OPT_FALLBACK;
+    const int32_t before = out->cert.n_launches;
+    rc = ray_fallback(p, &oc, &out->cert);
+    out->n_launches += out->cert.n_launches - before;
+    return rc;
 }
 
 #ifdef ENUMGPU_TRACE

@@ -150,8 +150,8 @@ k_independent(const LaunchParams prm, BlockPartial* __restrict__ partials)
             else if (st == 1) ++ni;
             else {
                 ++nf;
-                if (prm.list_count) list_append(prm.list_count, prm.list_ranks, prm.list_cap, r);
                 const double key = prm.maximize ? -z : z;
+                if (prm.list_count && in_window(key, prm.list_key_max)) list_append(prm.list_count, prm.list_ranks, prm.list_cap, r);
                 if (better(key, r, best_key, best_rank)) { best_key = key; best_rank = r; }
             }
             next_subset_regs<M>(S, n);
@@ -198,8 +198,8 @@ k_independent_generic(const LaunchParams prm, BlockPartial* __restrict__ partial
             else if (st == 1) ++ni;
             else {
                 ++nf;
-                if (prm.list_count) list_append(prm.list_count, prm.list_ranks, prm.list_cap, r);
                 const double key = prm.maximize ? -z : z;
+                if (prm.list_count && in_window(key, prm.list_key_max)) list_append(prm.list_count, prm.list_ranks, prm.list_cap, r);
                 if (better(key, r, best_key, best_rank)) { best_key = key; best_rank = r; }
             }
             int i = m - 1;
