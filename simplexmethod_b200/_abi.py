@@ -153,7 +153,11 @@ SYMBOLS = {
                                          C.c_double, C.POINTER(Certificate)]),
     "enumgpu_certify_optimum": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result), C.c_double,
                                            C.c_uint64, C.POINTER(Optimum)]),
+    "enumgpu_solve_objectives": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.c_int32, C.POINTER(C.c_double),
+                                            C.c_int32, C.c_uint64, C.POINTER(Result)]),
 }
+
+MAX_OBJECTIVES = 1 << 20
 
 
 def bind(lib, symbols=SYMBOLS):

@@ -41,7 +41,7 @@ public:
     EnumerationSolver(const EnumerationSolver& o)
         : problem_(o.problem_), devices_(o.devices_), algo_(o.algo_), rule_(o.rule_), eps_feas_(o.eps_feas_), eps_piv_(o.eps_piv_),
           rank_begin_(o.rank_begin_), rank_end_(o.rank_end_), check_unbounded_(o.check_unbounded_), optimal_duals_(o.optimal_duals_),
-          res_(o.res_), cert_(o.cert_), cert_basis_(o.cert_basis_), solved_(o.solved_), certified_(o.certified_) {}   // handles are not shared
+          res_(o.res_), obj_res_(o.obj_res_), cert_(o.cert_), cert_basis_(o.cert_basis_), solved_(o.solved_), certified_(o.certified_) {}   // handles are not shared
     EnumerationSolver& operator=(const EnumerationSolver&) = delete;
 
     // optional knobs (not in the reference)
@@ -86,6 +86,34 @@ public:
         for (int j = 0; j < n_orig; ++j) head[j] = x[j];
         return head;
     }
+
+    // solve() for every column of C (n x k, one cost vector per column, the problem's sense for all of them) with one
+    // enumeration (enumgpu_solve_objectives, current device): element i is what solve() returns with c = column i.
+    // Same exceptions as solve(); objectiveResults() then holds the k result structs.  Honours the rank range.
+    std::vector<Eigen::VectorXd> solveObjectives(const Eigen::MatrixXd& C)
+    {
+        const enumgpu_problem p = problemStruct();
+        if (C.rows() != p.n || C.cols() < 1)
+            throw std::invalid_argument("EnumerationSolver: solveObjectives needs an n x k matrix of cost vectors, k >= 1");
+        enumgpu_options o = options();
+        o.rank_begin = rank_begin_; o.rank_end = rank_end_;
+        obj_res_.assign(static_cast<size_t>(C.cols()), enumgpu_result{});
+        const int rc = enumgpu_solve_objectives(&p, &o, static_cast<int32_t>(C.cols()), C.data(), p.n, 0, obj_res_.data());
+        if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
+        if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
+        const int n_orig = problem_.GetOriginalVariablesCount();
+        std::vector<Eigen::VectorXd> xs;
+        for (const enumgpu_result& r : obj_res_) {
+            if (r.status == ENUMGPU_NO_FEASIBLE) throw std::runtime_error("the problem has no feasible basic solution");
+            Eigen::VectorXd x = Eigen::VectorXd::Zero(p.n);
+            for (int i = 0; i < r.m; ++i) x[r.basis[i]] = r.x_B[i];
+            Eigen::VectorXd head(n_orig);
+            for (int j = 0; j < n_orig; ++j) head[j] = x[j];
+            xs.push_back(head);
+        }
+        return xs;
+    }
+    const std::vector<enumgpu_result>& objectiveResults() const { return obj_res_; }
 
     // what the parity metric needs; valid after solve() (also after a "no feasible basis" throw)
     std::vector<int> optimalBasis() const { need(); return std::vector<int>(res_.basis, res_.basis + res_.m); }
@@ -194,6 +222,7 @@ private:
                               enumgpu_optimum*);
     OptimumFn optimal_duals_ = nullptr;        // &enumgpu_certify_optimum when setOptimalDuals(true)
     enumgpu_result res_{};
+    std::vector<enumgpu_result> obj_res_;      // solveObjectives(), one per cost vector
     enumgpu_certificate cert_{};
     std::vector<int> cert_basis_;
     int cert_source_ = ENUMGPU_OPT_WINNER;

@@ -19,6 +19,7 @@
 #include "enum_common.cuh"
 #include "k_independent.cuh"
 #include "k_shared.cuh"
+#include "k_objectives.cuh"
 
 using namespace enumgpu;
 
@@ -1171,6 +1172,211 @@ extern "C" int enumgpu_eval_ranks(const enumgpu_problem* p, const enumgpu_option
     rc = body();
     cudaStreamDestroy(st);
     return rc;
+}
+
+// ------------------------------------------------------------------ many objectives over one feasible set (DESIGN.md §3.2)
+
+constexpr int32_t  kMaxObjectives = 1 << 20;
+constexpr uint32_t kObjChunk = 1u << 21;      // listed bases per k_obj_values + k_objectives pass (chunk buffers: 9 B/row)
+
+struct ObjPass {
+    enumgpu_problem dp;                       // device copy, A packed (lda = m)
+    const uint64_t* binom;
+    const double* C;                          // device, cost vector i at C[i * n]
+    int32_t k;
+    int W;                                    // objectives per block (power of two <= kObjThreads)
+    dim3 grid;                                // slices x objective tiles
+    uint8_t* S;                               // chunk buffers, [m][chunk]
+    double* x;
+    Best* best;                               // [slices][k]
+    cudaStream_t st;
+};
+
+// x_B of `count` listed ranks, then their keys under every cost vector: 2 launches
+template <int M>
+static cudaError_t objectives_chunk(const ObjPass& a, const uint64_t* ranks, uint32_t count, int first)
+{
+    const int n = a.dp.n;
+    const unsigned blocks = (count + kObjThreads - 1) / kObjThreads;
+    if constexpr (M <= 12) {
+        const size_t smem = (size_t)(n * M + M + n) * sizeof(double) + sizeof(uint64_t) * kBinomRows * kBinomCols;
+        k_obj_values<M><<<blocks, kObjThreads, smem, a.st>>>(a.dp.A_colmajor, a.dp.b, a.binom, n, ranks, count, a.S, a.x);
+    } else {
+        k_obj_values_generic<<<blocks, kObjThreads, 0, a.st>>>(a.dp.A_colmajor, a.dp.b, a.binom, M, n, ranks, count, a.S, a.x);
+    }
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const size_t smem = (size_t)M * kObjTile * (sizeof(double) + 1) + kObjTile * sizeof(uint64_t) + (size_t)n * a.W * sizeof(double);
+    e = cudaFuncSetAttribute(k_objectives<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    k_objectives<M><<<a.grid, kObjThreads, smem, a.st>>>(a.S, a.x, ranks, count, n, a.dp.maximize ? 1 : 0, a.C, a.k, a.W, first,
+                                                          a.best);
+    return cudaGetLastError();
+}
+
+static cudaError_t dispatch_objectives(const ObjPass& a, const uint64_t* ranks, uint32_t count, int first)
+{
+    switch (a.dp.m) {
+#define ENUMGPU_CASE(M_) case M_: return objectives_chunk<M_>(a, ranks, count, first);
+        ENUMGPU_CASE(1) ENUMGPU_CASE(2) ENUMGPU_CASE(3) ENUMGPU_CASE(4)
+        ENUMGPU_CASE(5) ENUMGPU_CASE(6) ENUMGPU_CASE(7) ENUMGPU_CASE(8)
+        ENUMGPU_CASE(9) ENUMGPU_CASE(10) ENUMGPU_CASE(11) ENUMGPU_CASE(12)
+        ENUMGPU_CASE(13) ENUMGPU_CASE(14) ENUMGPU_CASE(15) ENUMGPU_CASE(16)
+#undef ENUMGPU_CASE
+    }
+    return cudaErrorInvalidValue;
+}
+
+extern "C" int enumgpu_solve_objectives(const enumgpu_problem* p, const enumgpu_options* o, int32_t k, const double* C,
+                                        int32_t ldc, uint64_t max_list, enumgpu_result* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "solve_objectives: out is NULL");
+    if (k < 1 || k > kMaxObjectives) return fail(ENUMGPU_ERR_ARG, "solve_objectives: k=%d outside 1..%d", k, kMaxObjectives);
+    memset(out, 0, sizeof(enumgpu_result) * (size_t)k);
+    auto all = [&](int rc) { for (int32_t i = 0; i < k; ++i) out[i].status = rc; return rc; };
+    if (!p) return all(fail(ENUMGPU_ERR_ARG, "problem is NULL"));
+    if (!C) return all(fail(ENUMGPU_ERR_ARG, "solve_objectives: C is NULL"));
+    if (ldc < p->n) return all(fail(ENUMGPU_ERR_ARG, "solve_objectives: ldc=%d < n=%d", ldc, p->n));
+    if (o && (o->shard_index != 0 || o->shard_count != 0))
+        return all(fail(ENUMGPU_ERR_ARG, "solve_objectives: shards are not supported (split the range with enumgpu_shard_begin)"));
+    enumgpu_problem q = *p;
+    q.c = C;                                  // p->c is not read; column 0 stands in where the enumeration wants a c
+    Resolved rs;
+    int rc = resolve(&q, o, &rs, true);
+    if (rc) return all(rc);
+    const int m = p->m, n = p->n;
+    for (int32_t i = 0; i < k; ++i)
+        for (int j = 0; j < n; ++j)
+            if (!std::isfinite(C[j + (size_t)i * ldc])) return all(fail(ENUMGPU_ERR_NONFINITE, "C(%d,%d) is not finite", j, i));
+    if (enumgpu_device_count() < 1) return all(fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)"));
+    if (max_list == 0) max_list = 1ull << 26;
+    // the list never holds more than the range has ranks
+    const uint64_t span = rs.end - rs.begin, cap = std::max<uint64_t>(1, std::min(max_list, span));
+    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, cap);
+
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    keep_pool_memory(dev);
+    cudaStream_t st = nullptr;
+    if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess)
+        return all(fail(ENUMGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(cudaGetLastError())));
+    std::vector<enumgpu_partial> acc((size_t)k), recs((size_t)k);
+    int32_t launches = 0;
+    float ms = 0.f;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    auto body = [&]() -> int {
+        DeviceProblem D;
+        int r2 = upload_problem(&q, st, &D);
+        if (r2) return r2;
+        ObjPass a;
+        a.dp = D.dp;
+        if ((r2 = device_binom(dev, &a.binom))) return r2;
+        std::vector<double> hC((size_t)k * n);
+        for (int32_t i = 0; i < k; ++i) memcpy(&hC[(size_t)i * n], C + (size_t)i * ldc, sizeof(double) * n);
+        a.k = k;
+        a.W = 1;
+        while (a.W < k && a.W < kObjThreads) a.W *= 2;
+        const uint32_t tiles = (uint32_t)((k + a.W - 1) / a.W);
+        const uint32_t slices = std::max<uint32_t>(1, (uint32_t)(4 * sms) / tiles);
+        a.grid = dim3(slices, tiles);
+        a.st = st;
+        StreamBuf b_C, b_list, b_count, b_part, b_S, b_x, b_best, b_rec;
+        CU(b_C.alloc(hC.size() * sizeof(double), st));
+        CU(b_list.alloc(cap * sizeof(uint64_t), st));
+        CU(b_count.alloc(sizeof(unsigned long long), st));
+        CU(b_part.alloc(sizeof(enumgpu_partial), st));
+        CU(b_S.alloc((size_t)chunk * m, st));
+        CU(b_x.alloc((size_t)chunk * m * sizeof(double), st));
+        CU(b_best.alloc((size_t)slices * k * sizeof(Best), st));
+        CU(b_rec.alloc((size_t)k * sizeof(enumgpu_partial), st));
+        CU(cudaMemcpyAsync(b_C.p, hC.data(), hC.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        a.C = b_C.as<double>(); a.S = b_S.as<uint8_t>(); a.x = b_x.as<double>(); a.best = b_best.as<Best>();
+        CU(cudaEventCreate(&e0));
+        CU(cudaEventCreate(&e1));
+        CU(cudaEventRecord(e0, st));
+
+        // the feasible ranks of [lo, hi) into b_list (all of them if *count <= cap) and the range's record
+        auto list = [&](uint64_t lo, uint64_t hi, enumgpu_partial* lp, uint64_t* count) -> int {
+            CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
+            int32_t nl = 0;
+            const int r3 = enqueue_range(&D.dp, D.scale, rs, lo, hi, 0, 1, st, b_part.as<enumgpu_partial>(), &nl, nullptr,
+                                         b_count.as<unsigned long long>(), b_list.as<uint64_t>(), cap, INFINITY);
+            if (r3) return r3;
+            launches += nl;
+            unsigned long long h = 0;
+            CU(cudaMemcpyAsync(lp, b_part.p, sizeof *lp, cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(&h, b_count.p, sizeof h, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            *count = h;
+            return 0;
+        };
+        // every objective's best over the listed ranks, merged into acc with the range's counters
+        bool have = false;
+        auto absorb = [&](const enumgpu_partial& lp, uint64_t count) -> int {
+            for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
+                CU(dispatch_objectives(a, b_list.as<uint64_t>() + c0, (uint32_t)std::min<uint64_t>(chunk, count - c0), c0 == 0));
+                launches += 2;
+            }
+            k_obj_finish<<<(unsigned)((k + kObjThreads - 1) / kObjThreads), kObjThreads, 0, st>>>(
+                a.best, count ? (int)slices : 0, D.dp.A_colmajor, D.dp.b, a.C, a.binom, m, n, k, b_rec.as<enumgpu_partial>());
+            CU(cudaGetLastError());
+            ++launches;
+            CU(cudaMemcpyAsync(recs.data(), b_rec.p, (size_t)k * sizeof(enumgpu_partial), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            for (int32_t i = 0; i < k; ++i) {
+                enumgpu_partial& r = recs[i];
+                r.n_bases = lp.n_bases; r.n_singular = lp.n_singular; r.n_infeasible = lp.n_infeasible; r.n_feasible = lp.n_feasible;
+                r.algo_used = lp.algo_used;
+                if (have) enumgpu_merge_partial(&acc[i], &r);
+                else acc[i] = r;
+            }
+            have = true;
+            return 0;
+        };
+        enumgpu_partial lp;
+        uint64_t count = 0;
+        if ((r2 = list(rs.begin, rs.end, &lp, &count))) return r2;
+        if (count <= cap) {
+            if ((r2 = absorb(lp, count))) return r2;
+        } else {
+            // more feasible bases than the list holds: contiguous sub-ranges of about cap / 2 expected feasible bases
+            // each, and one that still overflows is halved.  Disjoint ranges merge exactly (enumgpu_merge_partial).
+            const uint64_t per = std::max<uint64_t>(1, cap / 2), parts = std::min(span, (count + per - 1) / per);
+            std::vector<std::pair<uint64_t, uint64_t>> todo;            // a stack: ascending ranges from its back
+            for (uint64_t i = parts; i-- > 0;)
+                todo.emplace_back(rs.begin + (uint64_t)((unsigned __int128)span * i / parts),
+                                  rs.begin + (uint64_t)((unsigned __int128)span * (i + 1) / parts));
+            while (!todo.empty()) {
+                const auto [lo, hi] = todo.back();
+                todo.pop_back();
+                if ((r2 = list(lo, hi, &lp, &count))) return r2;
+                if (count <= cap) {
+                    if ((r2 = absorb(lp, count))) return r2;
+                    continue;
+                }
+                const uint64_t mid = lo + (hi - lo) / 2;                 // a single rank never overflows: cap >= 1
+                todo.emplace_back(mid, hi);
+                todo.emplace_back(lo, mid);
+            }
+        }
+        CU(cudaEventRecord(e1, st));
+        CU(cudaStreamSynchronize(st));
+        CU(cudaEventElapsedTime(&ms, e0, e1));
+        return 0;
+    };
+    rc = body();
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    cudaStreamDestroy(st);
+    if (rc) return all(rc);
+    for (int32_t i = 0; i < k; ++i) {
+        enumgpu_partial_to_result(&acc[i], &out[i]);
+        out[i].kernel_ms = ms;
+        out[i].n_launches = launches;
+    }
+    return ENUMGPU_OK;
 }
 
 // ------------------------------------------------------------------ self-test of the branch-free reciprocal

@@ -260,6 +260,38 @@ class EnumerationSolver:
         self._cert = self._cert_basis = None
         return res
 
+    # -- many cost vectors over one feasible set (enumgpu_solve_objectives) ----------------------
+    def enumerateObjectives(self, costs, rank_begin: int = 0, rank_end: int = 0, max_list: int = 0):
+        """The raw result structs of every cost vector, from one enumeration: costs is a (k, n) array whose rows are
+        cost vectors (the problem's own sense for all of them; the problem's c is not used).  Entry i is what
+        enumerate() returns for the problem with c = costs[i], bit for bit; kernel_ms and n_launches describe the
+        whole call.  Runs on the current CUDA device.  max_list: feasible ranks held on the device (0 = 2^26)."""
+        p = self._problem
+        A = p.GetConstraintsMatrix()
+        n = A.shape[1]
+        costs = np.ascontiguousarray(np.asarray(costs, dtype=np.float64))   # C-contiguous (k, n) = column-major n x k
+        if costs.ndim != 2 or costs.shape[1] != n:
+            raise ValueError(f"costs must be a (k, {n}) array, one cost vector per row; got shape {costs.shape}")
+        k = costs.shape[0]
+        ps = _problem_struct(A, p.GetRightHandSide(), p.GetObjectiveCoefficients(), p.IsMaximization())
+        out = (_abi.Result * max(k, 1))()
+        _check(lib().enumgpu_solve_objectives(C.byref(ps), C.byref(self._options(rank_begin, rank_end)), k,
+                                              costs.ctypes.data_as(C.POINTER(C.c_double)), n, int(max_list), out))
+        return [out[i] for i in range(k)]
+
+    def solveObjectives(self, costs, rank_begin: int = 0, rank_end: int = 0) -> np.ndarray:
+        """solve() for every row of costs (a (k, n) array of cost vectors) with one enumeration: row i of the
+        (k, GetOriginalVariablesCount()) result is what solve() returns with c = costs[i].  Raises RuntimeError if
+        some cost vector has no optimum (no feasible basis), as solve() does."""
+        res = self.enumerateObjectives(costs, rank_begin, rank_end)
+        n = self._problem.GetObjectiveCoefficients().size
+        X = np.zeros((len(res), n))
+        for i, r in enumerate(res):
+            if r.status == _abi.NO_FEASIBLE:
+                raise RuntimeError("the problem has no feasible basic solution")
+            X[i, list(r.basis)[:r.m]] = list(r.x_B)[:r.m]
+        return X[:, : self._problem.GetOriginalVariablesCount()].copy()
+
     # -- certificate of the optimum: duals, reduced costs, unboundedness (enumgpu_certify) --------
     def _device_options(self):
         """Options for the handle-free entries: the solver's device list, tolerances, kernel and rule."""
