@@ -136,6 +136,71 @@ extern "C" int enumgpu_device_count(void)
     return n;
 }
 
+// the solve entries call this after checking their arguments (no CPU fallback); *count = the number of devices
+static int require_device(int* count = nullptr)
+{
+    const int n = enumgpu_device_count();
+    if (count) *count = n;
+    return n < 1 ? fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)") : 0;
+}
+
+// ------------------------------------------------------ per-call streams and buffers
+
+// Stream-ordered device buffer that returns itself to the pool when it goes out of scope — on the
+// error paths too (the free is enqueued behind the kernels that use the buffer).
+struct StreamBuf {
+    void* p = nullptr;
+    cudaStream_t st = nullptr;
+    StreamBuf() = default;
+    StreamBuf(const StreamBuf&) = delete;
+    StreamBuf& operator=(const StreamBuf&) = delete;
+    ~StreamBuf() { if (p) cudaFreeAsync(p, st); }
+    cudaError_t alloc(size_t bytes, cudaStream_t s) { st = s; return cudaMallocAsync(&p, bytes, s); }
+    template <class T> T* as() const { return static_cast<T*>(p); }
+};
+
+// Stream-ordered allocations come from the device's default memory pool.  Its
+// default release threshold (0) hands memory back to the OS at every
+// synchronisation, which makes each solve pay a fresh OS allocation; keep it.
+static void keep_pool_memory(int dev)
+{
+    static const bool enabled = [] { const char* e = getenv("ENUMGPU_KEEP_POOL"); return !(e && e[0] == '0'); }();
+    if (!enabled) return;
+    cudaMemPool_t pool;
+    if (cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
+        uint64_t thr = UINT64_MAX;
+        cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
+    } else cudaGetLastError();
+}
+
+// The stream of one handle-free call on the current device: a non-blocking stream of its own, or the caller's,
+// and with `timed` the two events of kernel_ms.  The destructor destroys what open() created, so declare it
+// before the call's StreamBufs: they queue their frees on its stream while that still exists.
+struct CallStream {
+    int dev = 0;
+    cudaStream_t st = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    bool own = false;
+    CallStream() = default;
+    CallStream(const CallStream&) = delete;
+    CallStream& operator=(const CallStream&) = delete;
+    ~CallStream()
+    {
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+        if (own) cudaStreamDestroy(st);
+    }
+    int open(bool timed, cudaStream_t caller = nullptr)
+    {
+        cudaGetDevice(&dev);
+        keep_pool_memory(dev);
+        if (caller) st = caller;
+        else { CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)); own = true; }
+        if (timed) { CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1)); }
+        return 0;
+    }
+};
+
 // ---------------------------------------------------------- service kernels
 
 // max |A_ij| -> *out   (one block)
@@ -375,12 +440,14 @@ extern "C" double enumgpu_fp64_peak_detail(int32_t repeats, double* detail)
         return -1.0;
     }
     if (repeats < 1) repeats = 3;
-    double* d = nullptr;
-    cudaEvent_t e0, e1;
-    if (cudaMalloc(&d, 32) != cudaSuccess || cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess) {
+    CallStream cs;
+    StreamBuf b;
+    if (cs.open(true)) return -1.0;
+    if (b.alloc(32, cs.st) != cudaSuccess) {
         fail(ENUMGPU_ERR_CUDA, "fp64 peak probe: %s", cudaGetErrorString(cudaGetLastError()));
         return -1.0;
     }
+    double* d = b.as<double>();
     double best = 0.0;
     const struct { int chains, threads, blocks_per_sm; } cfg[] = {{4, 512, 1}, {8, 512, 1}, {8, 256, 4}, {4, 512, 2}};
     for (const auto& c : cfg) {
@@ -388,14 +455,14 @@ extern "C" double enumgpu_fp64_peak_detail(int32_t repeats, double* detail)
         // ~6e7 cycles of FP64 pipe per launch: iters * 16 * chains DFMA per thread, 2 cycles per warp-DFMA per sub-core
         const int iters = (int)(6.0e7 / (16.0 * c.chains * 2.0 * (c.threads / 128) * c.blocks_per_sm));
         for (int r = 0; r < repeats + 1; ++r) {
-            cudaEventRecord(e0);
+            cudaEventRecord(cs.e0, cs.st);
             unsigned long long* clk = reinterpret_cast<unsigned long long*>(d + 1);
-            if (c.chains == 4) k_dfma_peak<4><<<blocks, c.threads>>>(d, iters, 1.0000001, 1e-9, clk);
-            else k_dfma_peak<8><<<blocks, c.threads>>>(d, iters, 1.0000001, 1e-9, clk);
-            cudaEventRecord(e1);
-            if (cudaEventSynchronize(e1) != cudaSuccess) { fail(ENUMGPU_ERR_CUDA, "fp64 peak probe: %s", cudaGetErrorString(cudaGetLastError())); best = -1.0; break; }
+            if (c.chains == 4) k_dfma_peak<4><<<blocks, c.threads, 0, cs.st>>>(d, iters, 1.0000001, 1e-9, clk);
+            else k_dfma_peak<8><<<blocks, c.threads, 0, cs.st>>>(d, iters, 1.0000001, 1e-9, clk);
+            cudaEventRecord(cs.e1, cs.st);
+            if (cudaEventSynchronize(cs.e1) != cudaSuccess) { fail(ENUMGPU_ERR_CUDA, "fp64 peak probe: %s", cudaGetErrorString(cudaGetLastError())); best = -1.0; break; }
             float ms = 0.f;
-            cudaEventElapsedTime(&ms, e0, e1);
+            cudaEventElapsedTime(&ms, cs.e0, cs.e1);
             const double flops = 2.0 * 16.0 * c.chains * (double)iters * (double)blocks * c.threads;
             const double tf = flops / (ms * 1e-3) * 1e-12;
             if (r > 0 && tf > best) {
@@ -410,40 +477,12 @@ extern "C" double enumgpu_fp64_peak_detail(int32_t repeats, double* detail)
         }
         if (best < 0) break;
     }
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(d);
     return best;
 }
 
 extern "C" double enumgpu_fp64_peak_tflops(int32_t repeats) { return enumgpu_fp64_peak_detail(repeats, nullptr); }
 
 // ------------------------------------------------------------ launch logic
-
-// Stream-ordered device buffer that returns itself to the pool when it goes out of scope — on the
-// error paths too (the free is enqueued behind the kernels that use the buffer).
-struct StreamBuf {
-    void* p = nullptr;
-    cudaStream_t st = nullptr;
-    StreamBuf() = default;
-    StreamBuf(const StreamBuf&) = delete;
-    StreamBuf& operator=(const StreamBuf&) = delete;
-    ~StreamBuf() { if (p) cudaFreeAsync(p, st); }
-    cudaError_t alloc(size_t bytes, cudaStream_t s) { st = s; return cudaMallocAsync(&p, bytes, s); }
-    template <class T> T* as() const { return static_cast<T*>(p); }
-};
-
-// Stream-ordered allocations come from the device's default memory pool.  Its
-// default release threshold (0) hands memory back to the OS at every
-// synchronisation, which makes each solve pay a fresh OS allocation; keep it.
-static void keep_pool_memory(int dev)
-{
-    static const bool enabled = [] { const char* e = getenv("ENUMGPU_KEEP_POOL"); return !(e && e[0] == '0'); }();
-    if (!enabled) return;
-    cudaMemPool_t pool;
-    if (cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
-        uint64_t thr = UINT64_MAX;
-        cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
-    } else cudaGetLastError();
-}
 
 template <int M>
 static cudaError_t launch_independent(const LaunchParams& prm, BlockPartial* parts, uint32_t blocks, cudaStream_t st)
@@ -562,6 +601,39 @@ struct Resolved {       // options with defaults applied and the range checked
     uint32_t shard_index, shard_count;
 };
 
+// pivot_rule, eps_feas and eps_piv of the options, defaults applied (the default eps_piv depends on the rule and m)
+static int resolve_tolerances(const enumgpu_options* o, int m, Resolved* r)
+{
+    r->rule = o ? o->pivot_rule : ENUMGPU_PIVOT_ABSOLUTE;
+    if (r->rule != ENUMGPU_PIVOT_ABSOLUTE && r->rule != ENUMGPU_PIVOT_RELATIVE) return fail(ENUMGPU_ERR_ARG, "unknown pivot_rule %d", r->rule);
+    r->eps_feas = (o && o->eps_feas >= 0) ? o->eps_feas : 1e-9;
+    r->eps_piv = (o && o->eps_piv >= 0) ? o->eps_piv : (r->rule == ENUMGPU_PIVOT_RELATIVE ? (double)m * 0x1p-52 : 1e-9);
+    // -0.0 passes the tests above and means 0.  Store +0.0: k_shared classifies leaf components by the high word of
+    // -eps_feas, whose sign bit must be set (with -(-0.0) = +0.0 every positive component would count as negative).
+    if (r->eps_feas == 0.0) r->eps_feas = 0.0;
+    if (r->eps_piv == 0.0) r->eps_piv = 0.0;
+    return 0;
+}
+
+static double resolve_eps_opt(double eps_opt)
+{
+    if (!(eps_opt >= 0)) return 1e-9;                    // negative (or NaN): the default
+    return eps_opt == 0.0 ? 0.0 : eps_opt;               // -0.0 means 0
+}
+
+// A, b and c of a problem in host memory are finite
+static int check_finite(const enumgpu_problem* p)
+{
+    for (int j = 0; j < p->n; ++j) {
+        if (!std::isfinite(p->c[j])) return fail(ENUMGPU_ERR_NONFINITE, "c[%d] is not finite", j);
+        for (int i = 0; i < p->m; ++i)
+            if (!std::isfinite(p->A_colmajor[i + (size_t)j * p->lda])) return fail(ENUMGPU_ERR_NONFINITE, "A(%d,%d) is not finite", i, j);
+    }
+    for (int i = 0; i < p->m; ++i)
+        if (!std::isfinite(p->b[i])) return fail(ENUMGPU_ERR_NONFINITE, "b[%d] is not finite", i);
+    return 0;
+}
+
 static int resolve(const enumgpu_problem* p, const enumgpu_options* o, Resolved* r, bool host_ptrs)
 {
     if (!p) return fail(ENUMGPU_ERR_ARG, "problem is NULL");
@@ -572,14 +644,7 @@ static int resolve(const enumgpu_problem* p, const enumgpu_options* o, Resolved*
     if (p->lda < p->m) return fail(ENUMGPU_ERR_ARG, "lda=%d < m=%d", p->lda, p->m);
     r->total = binom_mk(p->n, p->m);
     if (r->total == 0) return fail(ENUMGPU_ERR_RANGE, "C(%d,%d) does not fit 63 bits", p->n, p->m);
-    r->rule = o ? o->pivot_rule : ENUMGPU_PIVOT_ABSOLUTE;
-    if (r->rule != ENUMGPU_PIVOT_ABSOLUTE && r->rule != ENUMGPU_PIVOT_RELATIVE) return fail(ENUMGPU_ERR_ARG, "unknown pivot_rule %d", r->rule);
-    r->eps_feas = (o && o->eps_feas >= 0) ? o->eps_feas : 1e-9;
-    r->eps_piv = (o && o->eps_piv >= 0) ? o->eps_piv : (r->rule == ENUMGPU_PIVOT_RELATIVE ? (double)p->m * 0x1p-52 : 1e-9);
-    // -0.0 passes the tests above and means 0.  Store +0.0: k_shared classifies leaf components by the high word of
-    // -eps_feas, whose sign bit must be set (with -(-0.0) = +0.0 every positive component would count as negative).
-    if (r->eps_feas == 0.0) r->eps_feas = 0.0;
-    if (r->eps_piv == 0.0) r->eps_piv = 0.0;
+    if (const int rc = resolve_tolerances(o, p->m, r)) return rc;
     r->begin = o ? o->rank_begin : 0;
     r->end = o ? o->rank_end : 0;
     if (r->begin == 0 && r->end == 0) r->end = r->total;
@@ -594,16 +659,59 @@ static int resolve(const enumgpu_problem* p, const enumgpu_options* o, Resolved*
     }
     r->algo = o ? o->algo : ENUMGPU_ALGO_AUTO;
     if (r->algo < ENUMGPU_ALGO_AUTO || r->algo > ENUMGPU_ALGO_SHARED) return fail(ENUMGPU_ERR_ARG, "unknown algo %d", r->algo);
-    if (host_ptrs) {
-        for (int j = 0; j < p->n; ++j) {
-            if (!std::isfinite(p->c[j])) return fail(ENUMGPU_ERR_NONFINITE, "c[%d] is not finite", j);
-            for (int i = 0; i < p->m; ++i)
-                if (!std::isfinite(p->A_colmajor[i + (size_t)j * p->lda])) return fail(ENUMGPU_ERR_NONFINITE, "A(%d,%d) is not finite", i, j);
-        }
-        for (int i = 0; i < p->m; ++i)
-            if (!std::isfinite(p->b[i])) return fail(ENUMGPU_ERR_NONFINITE, "b[%d] is not finite", i);
-    }
-    return 0;
+    return host_ptrs ? check_finite(p) : 0;
+}
+
+// the absolute rule's singularity threshold eps_piv * max|A_ij|; the relative rule tests each basis (thr = 0)
+static double pivot_threshold(const Resolved& rs, double scale)
+{
+    return rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * scale;
+}
+
+// The fields of the launch parameters that follow from the problem (device pointers) and the tolerances
+static LaunchParams problem_params(const enumgpu_problem* pd, const uint64_t* d_binom, const Resolved& rs, double scale)
+{
+    LaunchParams prm{};
+    prm.A = pd->A_colmajor; prm.b = pd->b; prm.c = pd->c; prm.binom = d_binom;
+    prm.m = pd->m; prm.n = pd->n; prm.lda = pd->lda; prm.maximize = pd->maximize ? 1 : 0;
+    prm.eps_feas = rs.eps_feas;
+    prm.pivot_rule = rs.rule;
+    prm.thr = pivot_threshold(rs, scale);
+    prm.rel_eps = rs.rule == ENUMGPU_PIVOT_RELATIVE ? rs.eps_piv : 0.0;
+    return prm;
+}
+
+// max|A_ij| of a problem in host memory
+static double max_abs_A(const enumgpu_problem* p)
+{
+    double s = 0.0;
+    for (int j = 0; j < p->n; ++j)
+        for (int i = 0; i < p->m; ++i) s = fmax(s, fabs(p->A_colmajor[i + (size_t)j * p->lda]));
+    return s;
+}
+
+// The packed copy of a problem that the device works on: A (lda = m), then b, then c
+static size_t packed_doubles(const enumgpu_problem* p) { return (size_t)p->m * p->n + p->m + p->n; }
+
+// packs host problem p into out[packed_doubles(p)]; returns max|A_ij|
+static double pack_problem(const enumgpu_problem* p, double* out)
+{
+    const int m = p->m, n = p->n;
+    for (int j = 0; j < n; ++j) memcpy(out + (size_t)j * m, p->A_colmajor + (size_t)j * p->lda, sizeof(double) * m);
+    memcpy(out + (size_t)m * n, p->b, sizeof(double) * m);
+    memcpy(out + (size_t)m * n + m, p->c, sizeof(double) * n);
+    return max_abs_A(p);
+}
+
+// p as it reads from its packed copy at d (device memory)
+static enumgpu_problem packed_view(const enumgpu_problem* p, const double* d)
+{
+    enumgpu_problem dp = *p;
+    dp.lda = p->m;
+    dp.A_colmajor = d;
+    dp.b = d + (size_t)p->m * p->n;
+    dp.c = dp.b + p->m;
+    return dp;
 }
 
 // Device scratch of one enqueue: the control block (zero on entry; the last block of the enqueue resets it) and
@@ -645,17 +753,26 @@ static int scratch_reserve(Scratch* sc, size_t n_parts, cudaStream_t st)
 // Checked once per process and device (a 4 M-operand run of the self-test, ~0.1 ms) before the shared kernel is
 // first used; on a mismatch — a toolkit or driver that expands the intrinsic differently — the library falls back
 // to the independent kernel (plain __drcp_rn) and says so in enumgpu_last_error().
-static int rcp_selftest_device(uint64_t n_operands, uint64_t seed, uint64_t* n_mismatch, double* first_bad, cudaStream_t st);
+static int rcp_selftest_device(uint64_t n_operands, uint64_t seed, uint64_t* n_mismatch, double* first_bad);
 static bool shared_rcp_trusted(int dev);
 
-// Enqueue everything for one rank range on one stream of the current device.
+// The listing of an enqueue (enumgpu_list_window): the feasible ranks whose key is at most key_max, appended in
+// arrival order; *count (device memory, zero on entry) counts all of them, ranks[0, cap) holds the first cap.
+struct Listing {
+    unsigned long long* count;
+    uint64_t* ranks;
+    uint64_t cap;
+    double key_max;
+};
+
+// Enqueue everything for the rank range and shard of rs on one stream of the current device.
 // scale_host < 0: max|A_ij| is computed on the device first (one synchronisation of st).
-static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Resolved& rs, uint64_t begin, uint64_t end,
-                         uint32_t shard_index, uint32_t shard_count,
-                         cudaStream_t st, enumgpu_partial* partial_dev, int32_t* n_launches, Scratch* scratch = nullptr,
-                         unsigned long long* list_count = nullptr, uint64_t* list_ranks = nullptr, uint64_t list_cap = 0,
-                         double list_key_max = INFINITY)
+static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Resolved& rs, cudaStream_t st,
+                         enumgpu_partial* partial_dev, int32_t* n_launches, Scratch* scratch = nullptr,
+                         const Listing* list = nullptr)
 {
+    const uint64_t begin = rs.begin, end = rs.end;
+    const uint32_t shard_index = rs.shard_index, shard_count = rs.shard_count;
     int launches = 0;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
@@ -679,16 +796,11 @@ static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Res
         CU(cudaStreamSynchronize(st));
     }
 
-    LaunchParams prm;
-    prm.A = pd->A_colmajor; prm.b = pd->b; prm.c = pd->c; prm.binom = d_binom;
-    prm.m = pd->m; prm.n = pd->n; prm.lda = pd->lda; prm.maximize = pd->maximize ? 1 : 0;
-    prm.eps_feas = rs.eps_feas;
-    prm.pivot_rule = rs.rule;
-    prm.thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * scale_host;
-    prm.rel_eps = rs.rule == ENUMGPU_PIVOT_RELATIVE ? rs.eps_piv : 0.0;
+    LaunchParams prm = problem_params(pd, d_binom, rs, scale_host);
     prm.rank_begin = begin; prm.rank_end = end; prm.chunk = 1;
     prm.shard_index = 0; prm.shard_count = 1;
-    prm.list_count = list_count; prm.list_ranks = list_ranks; prm.list_cap = list_cap; prm.list_key_max = list_key_max;
+    const Listing l = list ? *list : Listing{nullptr, nullptr, 0, INFINITY};
+    prm.list_count = l.count; prm.list_ranks = l.ranks; prm.list_cap = l.cap; prm.list_key_max = l.key_max;
     const bool first_shard = (shard_index == 0), last_shard = (shard_index + 1 == shard_count);
 
     int algo = rs.algo;
@@ -908,9 +1020,9 @@ extern "C" int enumgpu_enqueue_device(const enumgpu_problem* p_dev, double scale
     int rc = resolve(p_dev, o, &rs, false);
     if (rc) return rc;
     if (!partial_dev) return fail(ENUMGPU_ERR_ARG, "partial_dev is NULL");
-    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    if ((rc = require_device())) return rc;
     cudaStream_t st = o ? (cudaStream_t)o->stream : nullptr;
-    return enqueue_range(p_dev, scale_A, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, partial_dev, n_launches);
+    return enqueue_range(p_dev, scale_A, rs, st, partial_dev, n_launches);
 }
 
 extern "C" void enumgpu_partial_to_result(const enumgpu_partial* ph, enumgpu_result* out)
@@ -949,53 +1061,32 @@ extern "C" int enumgpu_eval_basis(const enumgpu_problem* p, const enumgpu_option
     if (!basis || !x_B || !objective || !basis_class) return fail(ENUMGPU_ERR_ARG, "eval_basis: NULL argument");
     const int m = p->m, n = p->n;
     if (m < 1 || n < 1 || p->lda < m) return fail(ENUMGPU_ERR_ARG, "eval_basis: bad dimensions m=%d n=%d lda=%d", m, n, p->lda);
-    const int rule = o ? o->pivot_rule : ENUMGPU_PIVOT_ABSOLUTE;
-    if (rule != ENUMGPU_PIVOT_ABSOLUTE && rule != ENUMGPU_PIVOT_RELATIVE) return fail(ENUMGPU_ERR_ARG, "unknown pivot_rule %d", rule);
-    const double eps_feas = (o && o->eps_feas >= 0) ? o->eps_feas : 1e-9;
-    const double eps_piv = (o && o->eps_piv >= 0) ? o->eps_piv : (rule == ENUMGPU_PIVOT_RELATIVE ? (double)m * 0x1p-52 : 1e-9);
+    Resolved rs{};
+    int rc = resolve_tolerances(o, m, &rs);
+    if (rc) return rc;
     for (int i = 0; i < m; ++i)
         if (basis[i] < 0 || basis[i] >= n) return fail(ENUMGPU_ERR_ARG, "basis index %d out of range", basis[i]);
-    double scale = 0.0;
-    for (int j = 0; j < n; ++j) {
-        if (!std::isfinite(p->c[j])) return fail(ENUMGPU_ERR_NONFINITE, "c[%d] is not finite", j);
-        for (int i = 0; i < m; ++i) {
-            const double v = p->A_colmajor[i + (size_t)j * p->lda];
-            if (!std::isfinite(v)) return fail(ENUMGPU_ERR_NONFINITE, "A(%d,%d) is not finite", i, j);
-            scale = fmax(scale, fabs(v));
-        }
-    }
-    for (int i = 0; i < m; ++i)
-        if (!std::isfinite(p->b[i])) return fail(ENUMGPU_ERR_NONFINITE, "b[%d] is not finite", i);
-    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    if ((rc = check_finite(p)) || (rc = require_device())) return rc;
     // gather (Canonical.cpp:183-187): W = [A(:, basis) | b] column-major, then c_B, then room for 1/pivot
     const size_t w_elems = (size_t)m * (m + 1);
     std::vector<double> stage(w_elems + 2 * (size_t)m);
     for (int j = 0; j < m; ++j) memcpy(&stage[(size_t)j * m], p->A_colmajor + (size_t)basis[j] * p->lda, sizeof(double) * m);
     memcpy(&stage[(size_t)m * m], p->b, sizeof(double) * m);
     for (int j = 0; j < m; ++j) stage[w_elems + j] = p->c[basis[j]];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    keep_pool_memory(dev);
-    cudaStream_t st = nullptr;
-    CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     std::vector<double> h_out((size_t)m + 2, 0.0);
-    auto body = [&]() -> int {
-        StreamBuf b_in, b_out;
-        CU(b_in.alloc(stage.size() * sizeof(double), st));
-        CU(b_out.alloc(h_out.size() * sizeof(double), st));
-        double* d_in = b_in.as<double>();
-        CU(cudaMemcpyAsync(d_in, stage.data(), stage.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-        CU(cudaMemsetAsync(b_out.p, 0, h_out.size() * sizeof(double), st));
-        k_eval_any<<<1, 256, 0, st>>>(d_in, d_in + w_elems, m, rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : eps_piv * scale, eps_feas,
-                                      rule, eps_piv, d_in + w_elems + m, b_out.as<double>());
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(h_out.data(), b_out.p, h_out.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        return 0;
-    };
-    const int rc = body();
-    cudaStreamDestroy(st);
-    if (rc) return rc;
+    CallStream cs;
+    StreamBuf b_in, b_out;
+    if ((rc = cs.open(false))) return rc;
+    CU(b_in.alloc(stage.size() * sizeof(double), cs.st));
+    CU(b_out.alloc(h_out.size() * sizeof(double), cs.st));
+    double* d_in = b_in.as<double>();
+    CU(cudaMemcpyAsync(d_in, stage.data(), stage.size() * sizeof(double), cudaMemcpyHostToDevice, cs.st));
+    CU(cudaMemsetAsync(b_out.p, 0, h_out.size() * sizeof(double), cs.st));
+    k_eval_any<<<1, 256, 0, cs.st>>>(d_in, d_in + w_elems, m, pivot_threshold(rs, max_abs_A(p)), rs.eps_feas, rs.rule, rs.eps_piv,
+                                     d_in + w_elems + m, b_out.as<double>());
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h_out.data(), b_out.p, h_out.size() * sizeof(double), cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaStreamSynchronize(cs.st));
     for (int i = 0; i < m; ++i) x_B[i] = h_out[i];
     *objective = h_out[m];
     *basis_class = (int32_t)h_out[m + 1];
@@ -1025,23 +1116,59 @@ struct DeviceProblem {
 };
 static int upload_problem(const enumgpu_problem* p, cudaStream_t st, DeviceProblem* out)
 {
-    const int m = p->m, n = p->n;
-    std::vector<double> stage((size_t)m * n + m + n);
-    for (int j = 0; j < n; ++j)
-        for (int i = 0; i < m; ++i) {
-            const double v = p->A_colmajor[i + (size_t)j * p->lda];
-            stage[(size_t)j * m + i] = v;
-            out->scale = fmax(out->scale, fabs(v));
-        }
-    memcpy(&stage[(size_t)m * n], p->b, sizeof(double) * m);
-    memcpy(&stage[(size_t)m * n + m], p->c, sizeof(double) * n);
+    std::vector<double> stage(packed_doubles(p));
+    out->scale = pack_problem(p, stage.data());
     CU(out->buf.alloc(stage.size() * sizeof(double), st));
     CU(cudaMemcpyAsync(out->buf.p, stage.data(), stage.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-    out->dp = *p;
-    out->dp.lda = m;
-    out->dp.A_colmajor = out->buf.as<double>();
-    out->dp.b = out->buf.as<double>() + (size_t)m * n;
-    out->dp.c = out->dp.b + m;
+    out->dp = packed_view(p, out->buf.as<double>());
+    return 0;
+}
+
+// The timed enumeration of a synchronous entry: record e0, enqueue the range of rs, record e1, then the record
+// (and the listing's count into *h_count) back to the host with one synchronisation, and the result into *out.
+static int enumerate_timed(const enumgpu_problem* pd, double scale, const Resolved& rs, const CallStream& cs,
+                           const Listing* list, unsigned long long* h_count, enumgpu_result* out)
+{
+    StreamBuf b_part;
+    CU(b_part.alloc(sizeof(enumgpu_partial), cs.st));
+    enumgpu_partial h_part;
+    int32_t launches = 0;
+    CU(cudaEventRecord(cs.e0, cs.st));
+    const int rc = enqueue_range(pd, scale, rs, cs.st, b_part.as<enumgpu_partial>(), &launches, nullptr, list);
+    if (rc) return rc;
+    CU(cudaEventRecord(cs.e1, cs.st));
+    CU(cudaMemcpyAsync(&h_part, b_part.p, sizeof h_part, cudaMemcpyDeviceToHost, cs.st));
+    if (list) CU(cudaMemcpyAsync(h_count, list->count, sizeof *h_count, cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaStreamSynchronize(cs.st));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    enumgpu_partial_to_result(&h_part, out);
+    out->kernel_ms = ms;
+    out->n_launches = launches;
+    return 0;
+}
+
+// The device part of list_window: *out, the count of the window, and the first `capacity` ranks, ascending.
+static int list_window_device(const enumgpu_problem* p, const Resolved& rs, double key_max, uint64_t* ranks, uint64_t capacity,
+                              std::vector<uint64_t>* fit, uint64_t* n_listed, enumgpu_result* out, uint64_t* n_window)
+{
+    CallStream cs;
+    DeviceProblem D;
+    StreamBuf b_count, b_ranks;
+    int rc;
+    if ((rc = cs.open(true)) || (rc = upload_problem(p, cs.st, &D))) return rc;
+    CU(b_count.alloc(sizeof(unsigned long long), cs.st));
+    CU(b_ranks.alloc(sizeof(uint64_t) * (capacity ? capacity : 1), cs.st));
+    CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), cs.st));
+    const Listing list{b_count.as<unsigned long long>(), b_ranks.as<uint64_t>(), capacity, key_max};
+    unsigned long long h_count = 0;
+    if ((rc = enumerate_timed(&D.dp, D.scale, rs, cs, &list, &h_count, out))) return rc;
+    const uint64_t k = h_count < capacity ? (uint64_t)h_count : capacity;
+    if (fit) { fit->resize(k); ranks = fit->data(); }
+    if (n_window) *n_window = h_count;
+    if (k) CU(cudaMemcpy(ranks, b_ranks.p, sizeof(uint64_t) * k, cudaMemcpyDeviceToHost));
+    *n_listed = k;
+    std::sort(ranks, ranks + k);             // the device appends in arrival order; hand them out ascending
     return 0;
 }
 
@@ -1057,55 +1184,9 @@ static int list_window(const enumgpu_problem* p, const enumgpu_options* o, doubl
     if (capacity && !ranks && !fit) return out->status = fail(ENUMGPU_ERR_ARG, "list_window: ranks is NULL but capacity is %llu", (unsigned long long)capacity);
     Resolved rs;
     int rc = resolve(p, o, &rs, true);
+    if (rc == 0) rc = require_device();
+    if (rc == 0) rc = list_window_device(p, rs, key_max, ranks, capacity, fit, n_listed, out, n_window);
     if (rc) return out->status = rc;
-    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
-    int dev = 0;
-    cudaGetDevice(&dev);
-    keep_pool_memory(dev);
-    cudaStream_t st = nullptr;
-    if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess)
-        return out->status = fail(ENUMGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(cudaGetLastError()));
-    enumgpu_partial h_part;
-    unsigned long long h_count = 0;
-    int32_t launches = 0;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    auto body = [&]() -> int {
-        DeviceProblem D;
-        int r2 = upload_problem(p, st, &D);
-        if (r2) return r2;
-        StreamBuf b_part, b_count, b_ranks;
-        CU(b_part.alloc(sizeof(enumgpu_partial), st));
-        CU(b_count.alloc(sizeof(unsigned long long), st));
-        CU(b_ranks.alloc(sizeof(uint64_t) * (capacity ? capacity : 1), st));
-        CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
-        CU(cudaEventCreate(&e0));
-        CU(cudaEventCreate(&e1));
-        CU(cudaEventRecord(e0, st));
-        r2 = enqueue_range(&D.dp, D.scale, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, b_part.as<enumgpu_partial>(),
-                           &launches, nullptr, b_count.as<unsigned long long>(), b_ranks.as<uint64_t>(), capacity, key_max);
-        if (r2) return r2;
-        CU(cudaEventRecord(e1, st));
-        CU(cudaMemcpyAsync(&h_part, b_part.p, sizeof h_part, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(&h_count, b_count.p, sizeof h_count, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        const uint64_t k = h_count < capacity ? (uint64_t)h_count : capacity;
-        if (fit) { fit->resize(k); ranks = fit->data(); }
-        if (n_window) *n_window = h_count;
-        if (k) CU(cudaMemcpy(ranks, b_ranks.p, sizeof(uint64_t) * k, cudaMemcpyDeviceToHost));
-        *n_listed = k;
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, e0, e1));
-        enumgpu_partial_to_result(&h_part, out);
-        out->kernel_ms = ms;
-        out->n_launches = launches;
-        return 0;
-    };
-    rc = body();
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    cudaStreamDestroy(st);
-    if (rc) return out->status = rc;
-    std::sort(ranks, ranks + *n_listed);     // the device appends in arrival order; hand them out ascending
     return out->status;
 }
 
@@ -1133,45 +1214,27 @@ extern "C" int enumgpu_eval_ranks(const enumgpu_problem* p, const enumgpu_option
     for (uint64_t i = 0; i < count; ++i)
         if (ranks[i] >= rs.total) return fail(ENUMGPU_ERR_RANGE, "eval_ranks: rank %llu out of range", (unsigned long long)ranks[i]);
     if (count > (1ull << 31)) return fail(ENUMGPU_ERR_RANGE, "eval_ranks: too many bases in one call");
-    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
-    int dev = 0;
-    cudaGetDevice(&dev);
-    keep_pool_memory(dev);
-    cudaStream_t st = nullptr;
-    CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    auto body = [&]() -> int {
-        DeviceProblem D;
-        int r2 = upload_problem(p, st, &D);
-        if (r2) return r2;
-        const int m = p->m;
-        StreamBuf b_ranks, b_x, b_z, b_cls;
-        const uint64_t* d_binom = nullptr;
-        r2 = device_binom(dev, &d_binom);
-        if (r2) return r2;
-        CU(b_ranks.alloc(sizeof(uint64_t) * count, st));
-        CU(b_x.alloc(sizeof(double) * count * m, st));
-        CU(b_z.alloc(sizeof(double) * count, st));
-        CU(b_cls.alloc(sizeof(int32_t) * count, st));
-        CU(cudaMemcpyAsync(b_ranks.p, ranks, sizeof(uint64_t) * count, cudaMemcpyHostToDevice, st));
-        LaunchParams prm{};
-        prm.A = D.dp.A_colmajor; prm.b = D.dp.b; prm.c = D.dp.c; prm.binom = d_binom;
-        prm.m = m; prm.n = p->n; prm.lda = m; prm.maximize = p->maximize ? 1 : 0;
-        prm.eps_feas = rs.eps_feas;
-        prm.pivot_rule = rs.rule;
-        prm.thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * D.scale;
-        prm.rel_eps = rs.rule == ENUMGPU_PIVOT_RELATIVE ? rs.eps_piv : 0.0;
-        const unsigned blocks = (unsigned)((count + 127) / 128);
-        k_eval_ranks<<<blocks, 128, 0, st>>>(prm, b_ranks.as<uint64_t>(), count, b_x.as<double>(), b_z.as<double>(), b_cls.as<int32_t>());
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(x_B, b_x.p, sizeof(double) * count * m, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(objective, b_z.p, sizeof(double) * count, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(basis_class, b_cls.p, sizeof(int32_t) * count, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        return 0;
-    };
-    rc = body();
-    cudaStreamDestroy(st);
-    return rc;
+    if ((rc = require_device())) return rc;
+    CallStream cs;
+    DeviceProblem D;
+    StreamBuf b_ranks, b_x, b_z, b_cls;
+    const uint64_t* d_binom = nullptr;
+    if ((rc = cs.open(false)) || (rc = upload_problem(p, cs.st, &D)) || (rc = device_binom(cs.dev, &d_binom))) return rc;
+    const int m = p->m;
+    CU(b_ranks.alloc(sizeof(uint64_t) * count, cs.st));
+    CU(b_x.alloc(sizeof(double) * count * m, cs.st));
+    CU(b_z.alloc(sizeof(double) * count, cs.st));
+    CU(b_cls.alloc(sizeof(int32_t) * count, cs.st));
+    CU(cudaMemcpyAsync(b_ranks.p, ranks, sizeof(uint64_t) * count, cudaMemcpyHostToDevice, cs.st));
+    const LaunchParams prm = problem_params(&D.dp, d_binom, rs, D.scale);
+    const unsigned blocks = (unsigned)((count + 127) / 128);
+    k_eval_ranks<<<blocks, 128, 0, cs.st>>>(prm, b_ranks.as<uint64_t>(), count, b_x.as<double>(), b_z.as<double>(), b_cls.as<int32_t>());
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(x_B, b_x.p, sizeof(double) * count * m, cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaMemcpyAsync(objective, b_z.p, sizeof(double) * count, cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaMemcpyAsync(basis_class, b_cls.p, sizeof(int32_t) * count, cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaStreamSynchronize(cs.st));
+    return 0;
 }
 
 // ------------------------------------------------------------------ many objectives over one feasible set (DESIGN.md §3.2)
@@ -1227,6 +1290,127 @@ static cudaError_t dispatch_objectives(const ObjPass& a, const uint64_t* ranks, 
     return cudaErrorInvalidValue;
 }
 
+// The device part of enumgpu_solve_objectives for q (c = column 0 of C) and the resolved options: out[0, k).
+static int solve_objectives_device(const enumgpu_problem* q, const Resolved& rs, int32_t k, const double* C, int32_t ldc,
+                                   uint64_t max_list, enumgpu_result* out)
+{
+    const int m = q->m, n = q->n;
+    if (max_list == 0) max_list = 1ull << 26;
+    // the list never holds more than the range has ranks
+    const uint64_t span = rs.end - rs.begin, cap = std::max<uint64_t>(1, std::min(max_list, span));
+    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, cap);
+
+    CallStream cs;
+    DeviceProblem D;
+    StreamBuf b_C, b_list, b_count, b_part, b_S, b_x, b_best, b_rec;
+    ObjPass a;
+    int rc;
+    if ((rc = cs.open(true)) || (rc = upload_problem(q, cs.st, &D)) || (rc = device_binom(cs.dev, &a.binom))) return rc;
+    const cudaStream_t st = cs.st;
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cs.dev);
+    std::vector<enumgpu_partial> acc((size_t)k), recs((size_t)k);
+    int32_t launches = 0;
+    a.dp = D.dp;
+    std::vector<double> hC((size_t)k * n);
+    for (int32_t i = 0; i < k; ++i) memcpy(&hC[(size_t)i * n], C + (size_t)i * ldc, sizeof(double) * n);
+    a.k = k;
+    a.W = 1;
+    while (a.W < k && a.W < kObjThreads) a.W *= 2;
+    const uint32_t tiles = (uint32_t)((k + a.W - 1) / a.W);
+    const uint32_t slices = std::max<uint32_t>(1, (uint32_t)(4 * sms) / tiles);
+    a.grid = dim3(slices, tiles);
+    a.st = st;
+    CU(b_C.alloc(hC.size() * sizeof(double), st));
+    CU(b_list.alloc(cap * sizeof(uint64_t), st));
+    CU(b_count.alloc(sizeof(unsigned long long), st));
+    CU(b_part.alloc(sizeof(enumgpu_partial), st));
+    CU(b_S.alloc((size_t)chunk * m, st));
+    CU(b_x.alloc((size_t)chunk * m * sizeof(double), st));
+    CU(b_best.alloc((size_t)slices * k * sizeof(Best), st));
+    CU(b_rec.alloc((size_t)k * sizeof(enumgpu_partial), st));
+    CU(cudaMemcpyAsync(b_C.p, hC.data(), hC.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    a.C = b_C.as<double>(); a.S = b_S.as<uint8_t>(); a.x = b_x.as<double>(); a.best = b_best.as<Best>();
+    CU(cudaEventRecord(cs.e0, st));
+
+    // the feasible ranks of [lo, hi) into b_list (all of them if *count <= cap) and the range's record
+    const Listing listing{b_count.as<unsigned long long>(), b_list.as<uint64_t>(), cap, INFINITY};
+    auto list = [&](uint64_t lo, uint64_t hi, enumgpu_partial* lp, uint64_t* count) -> int {
+        CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
+        Resolved sub = rs;
+        sub.begin = lo; sub.end = hi;
+        int32_t nl = 0;
+        const int r3 = enqueue_range(&D.dp, D.scale, sub, st, b_part.as<enumgpu_partial>(), &nl, nullptr, &listing);
+        if (r3) return r3;
+        launches += nl;
+        unsigned long long h = 0;
+        CU(cudaMemcpyAsync(lp, b_part.p, sizeof *lp, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&h, b_count.p, sizeof h, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        *count = h;
+        return 0;
+    };
+    // every objective's best over the listed ranks, merged into acc with the range's counters
+    bool have = false;
+    auto absorb = [&](const enumgpu_partial& lp, uint64_t count) -> int {
+        for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
+            CU(dispatch_objectives(a, b_list.as<uint64_t>() + c0, (uint32_t)std::min<uint64_t>(chunk, count - c0), c0 == 0));
+            launches += 2;
+        }
+        k_obj_finish<<<(unsigned)((k + kObjThreads - 1) / kObjThreads), kObjThreads, 0, st>>>(
+            a.best, count ? (int)slices : 0, D.dp.A_colmajor, D.dp.b, a.C, a.binom, m, n, k, b_rec.as<enumgpu_partial>());
+        CU(cudaGetLastError());
+        ++launches;
+        CU(cudaMemcpyAsync(recs.data(), b_rec.p, (size_t)k * sizeof(enumgpu_partial), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        for (int32_t i = 0; i < k; ++i) {
+            enumgpu_partial& r = recs[i];
+            r.n_bases = lp.n_bases; r.n_singular = lp.n_singular; r.n_infeasible = lp.n_infeasible; r.n_feasible = lp.n_feasible;
+            r.algo_used = lp.algo_used;
+            if (have) enumgpu_merge_partial(&acc[i], &r);
+            else acc[i] = r;
+        }
+        have = true;
+        return 0;
+    };
+    enumgpu_partial lp;
+    uint64_t count = 0;
+    if ((rc = list(rs.begin, rs.end, &lp, &count))) return rc;
+    if (count <= cap) {
+        if ((rc = absorb(lp, count))) return rc;
+    } else {
+        // more feasible bases than the list holds: contiguous sub-ranges of about cap / 2 expected feasible bases
+        // each, and one that still overflows is halved.  Disjoint ranges merge exactly (enumgpu_merge_partial).
+        const uint64_t per = std::max<uint64_t>(1, cap / 2), parts = std::min(span, (count + per - 1) / per);
+        std::vector<std::pair<uint64_t, uint64_t>> todo;            // a stack: ascending ranges from its back
+        for (uint64_t i = parts; i-- > 0;)
+            todo.emplace_back(rs.begin + (uint64_t)((unsigned __int128)span * i / parts),
+                              rs.begin + (uint64_t)((unsigned __int128)span * (i + 1) / parts));
+        while (!todo.empty()) {
+            const auto [lo, hi] = todo.back();
+            todo.pop_back();
+            if ((rc = list(lo, hi, &lp, &count))) return rc;
+            if (count <= cap) {
+                if ((rc = absorb(lp, count))) return rc;
+                continue;
+            }
+            const uint64_t mid = lo + (hi - lo) / 2;                 // a single rank never overflows: cap >= 1
+            todo.emplace_back(mid, hi);
+            todo.emplace_back(lo, mid);
+        }
+    }
+    CU(cudaEventRecord(cs.e1, st));
+    CU(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    for (int32_t i = 0; i < k; ++i) {
+        enumgpu_partial_to_result(&acc[i], &out[i]);
+        out[i].kernel_ms = ms;
+        out[i].n_launches = launches;
+    }
+    return ENUMGPU_OK;
+}
+
 extern "C" int enumgpu_solve_objectives(const enumgpu_problem* p, const enumgpu_options* o, int32_t k, const double* C,
                                         int32_t ldc, uint64_t max_list, enumgpu_result* out)
 {
@@ -1245,137 +1429,10 @@ extern "C" int enumgpu_solve_objectives(const enumgpu_problem* p, const enumgpu_
     Resolved rs;
     int rc = resolve(&q, o, &rs, true);
     if (rc) return all(rc);
-    const int m = p->m, n = p->n;
     for (int32_t i = 0; i < k; ++i)
-        for (int j = 0; j < n; ++j)
+        for (int j = 0; j < p->n; ++j)
             if (!std::isfinite(C[j + (size_t)i * ldc])) return all(fail(ENUMGPU_ERR_NONFINITE, "C(%d,%d) is not finite", j, i));
-    if (enumgpu_device_count() < 1) return all(fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)"));
-    if (max_list == 0) max_list = 1ull << 26;
-    // the list never holds more than the range has ranks
-    const uint64_t span = rs.end - rs.begin, cap = std::max<uint64_t>(1, std::min(max_list, span));
-    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, cap);
-
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    keep_pool_memory(dev);
-    cudaStream_t st = nullptr;
-    if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess)
-        return all(fail(ENUMGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(cudaGetLastError())));
-    std::vector<enumgpu_partial> acc((size_t)k), recs((size_t)k);
-    int32_t launches = 0;
-    float ms = 0.f;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    auto body = [&]() -> int {
-        DeviceProblem D;
-        int r2 = upload_problem(&q, st, &D);
-        if (r2) return r2;
-        ObjPass a;
-        a.dp = D.dp;
-        if ((r2 = device_binom(dev, &a.binom))) return r2;
-        std::vector<double> hC((size_t)k * n);
-        for (int32_t i = 0; i < k; ++i) memcpy(&hC[(size_t)i * n], C + (size_t)i * ldc, sizeof(double) * n);
-        a.k = k;
-        a.W = 1;
-        while (a.W < k && a.W < kObjThreads) a.W *= 2;
-        const uint32_t tiles = (uint32_t)((k + a.W - 1) / a.W);
-        const uint32_t slices = std::max<uint32_t>(1, (uint32_t)(4 * sms) / tiles);
-        a.grid = dim3(slices, tiles);
-        a.st = st;
-        StreamBuf b_C, b_list, b_count, b_part, b_S, b_x, b_best, b_rec;
-        CU(b_C.alloc(hC.size() * sizeof(double), st));
-        CU(b_list.alloc(cap * sizeof(uint64_t), st));
-        CU(b_count.alloc(sizeof(unsigned long long), st));
-        CU(b_part.alloc(sizeof(enumgpu_partial), st));
-        CU(b_S.alloc((size_t)chunk * m, st));
-        CU(b_x.alloc((size_t)chunk * m * sizeof(double), st));
-        CU(b_best.alloc((size_t)slices * k * sizeof(Best), st));
-        CU(b_rec.alloc((size_t)k * sizeof(enumgpu_partial), st));
-        CU(cudaMemcpyAsync(b_C.p, hC.data(), hC.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-        a.C = b_C.as<double>(); a.S = b_S.as<uint8_t>(); a.x = b_x.as<double>(); a.best = b_best.as<Best>();
-        CU(cudaEventCreate(&e0));
-        CU(cudaEventCreate(&e1));
-        CU(cudaEventRecord(e0, st));
-
-        // the feasible ranks of [lo, hi) into b_list (all of them if *count <= cap) and the range's record
-        auto list = [&](uint64_t lo, uint64_t hi, enumgpu_partial* lp, uint64_t* count) -> int {
-            CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
-            int32_t nl = 0;
-            const int r3 = enqueue_range(&D.dp, D.scale, rs, lo, hi, 0, 1, st, b_part.as<enumgpu_partial>(), &nl, nullptr,
-                                         b_count.as<unsigned long long>(), b_list.as<uint64_t>(), cap, INFINITY);
-            if (r3) return r3;
-            launches += nl;
-            unsigned long long h = 0;
-            CU(cudaMemcpyAsync(lp, b_part.p, sizeof *lp, cudaMemcpyDeviceToHost, st));
-            CU(cudaMemcpyAsync(&h, b_count.p, sizeof h, cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            *count = h;
-            return 0;
-        };
-        // every objective's best over the listed ranks, merged into acc with the range's counters
-        bool have = false;
-        auto absorb = [&](const enumgpu_partial& lp, uint64_t count) -> int {
-            for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
-                CU(dispatch_objectives(a, b_list.as<uint64_t>() + c0, (uint32_t)std::min<uint64_t>(chunk, count - c0), c0 == 0));
-                launches += 2;
-            }
-            k_obj_finish<<<(unsigned)((k + kObjThreads - 1) / kObjThreads), kObjThreads, 0, st>>>(
-                a.best, count ? (int)slices : 0, D.dp.A_colmajor, D.dp.b, a.C, a.binom, m, n, k, b_rec.as<enumgpu_partial>());
-            CU(cudaGetLastError());
-            ++launches;
-            CU(cudaMemcpyAsync(recs.data(), b_rec.p, (size_t)k * sizeof(enumgpu_partial), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            for (int32_t i = 0; i < k; ++i) {
-                enumgpu_partial& r = recs[i];
-                r.n_bases = lp.n_bases; r.n_singular = lp.n_singular; r.n_infeasible = lp.n_infeasible; r.n_feasible = lp.n_feasible;
-                r.algo_used = lp.algo_used;
-                if (have) enumgpu_merge_partial(&acc[i], &r);
-                else acc[i] = r;
-            }
-            have = true;
-            return 0;
-        };
-        enumgpu_partial lp;
-        uint64_t count = 0;
-        if ((r2 = list(rs.begin, rs.end, &lp, &count))) return r2;
-        if (count <= cap) {
-            if ((r2 = absorb(lp, count))) return r2;
-        } else {
-            // more feasible bases than the list holds: contiguous sub-ranges of about cap / 2 expected feasible bases
-            // each, and one that still overflows is halved.  Disjoint ranges merge exactly (enumgpu_merge_partial).
-            const uint64_t per = std::max<uint64_t>(1, cap / 2), parts = std::min(span, (count + per - 1) / per);
-            std::vector<std::pair<uint64_t, uint64_t>> todo;            // a stack: ascending ranges from its back
-            for (uint64_t i = parts; i-- > 0;)
-                todo.emplace_back(rs.begin + (uint64_t)((unsigned __int128)span * i / parts),
-                                  rs.begin + (uint64_t)((unsigned __int128)span * (i + 1) / parts));
-            while (!todo.empty()) {
-                const auto [lo, hi] = todo.back();
-                todo.pop_back();
-                if ((r2 = list(lo, hi, &lp, &count))) return r2;
-                if (count <= cap) {
-                    if ((r2 = absorb(lp, count))) return r2;
-                    continue;
-                }
-                const uint64_t mid = lo + (hi - lo) / 2;                 // a single rank never overflows: cap >= 1
-                todo.emplace_back(mid, hi);
-                todo.emplace_back(lo, mid);
-            }
-        }
-        CU(cudaEventRecord(e1, st));
-        CU(cudaStreamSynchronize(st));
-        CU(cudaEventElapsedTime(&ms, e0, e1));
-        return 0;
-    };
-    rc = body();
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    cudaStreamDestroy(st);
-    if (rc) return all(rc);
-    for (int32_t i = 0; i < k; ++i) {
-        enumgpu_partial_to_result(&acc[i], &out[i]);
-        out[i].kernel_ms = ms;
-        out[i].n_launches = launches;
-    }
+    if ((rc = require_device()) || (rc = solve_objectives_device(&q, rs, k, C, ldc, max_list, out))) return all(rc);
     return ENUMGPU_OK;
 }
 
@@ -1418,35 +1475,32 @@ k_rcp_selftest(uint64_t n, uint64_t seed, unsigned long long* n_bad, unsigned lo
     if (bad) atomicAdd(n_bad, bad);
 }
 
-static int rcp_selftest_device(uint64_t n_operands, uint64_t seed, uint64_t* n_mismatch, double* first_bad, cudaStream_t st)
+static int rcp_selftest_device(uint64_t n_operands, uint64_t seed, uint64_t* n_mismatch, double* first_bad)
 {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    unsigned long long* d = nullptr;
-    CU(cudaMalloc(&d, 16));
-    auto body = [&]() -> int {
-        CU(cudaMemsetAsync(d, 0, 16, st));
-        k_rcp_selftest<<<sms * 8, 256, 0, st>>>(n_operands, seed, d, d + 1);
-        CU(cudaGetLastError());
-        unsigned long long h[2] = {0, 0};
-        CU(cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        *n_mismatch = h[0];
-        if (first_bad) memcpy(first_bad, &h[1], 8);
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d);
-    return rc;
+    CallStream cs;
+    StreamBuf b;
+    if (const int rc = cs.open(false)) return rc;
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cs.dev);
+    CU(b.alloc(16, cs.st));
+    unsigned long long* d = b.as<unsigned long long>();
+    CU(cudaMemsetAsync(d, 0, 16, cs.st));
+    k_rcp_selftest<<<sms * 8, 256, 0, cs.st>>>(n_operands, seed, d, d + 1);
+    CU(cudaGetLastError());
+    unsigned long long h[2] = {0, 0};
+    CU(cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, cs.st));
+    CU(cudaStreamSynchronize(cs.st));
+    *n_mismatch = h[0];
+    if (first_bad) memcpy(first_bad, &h[1], 8);
+    return 0;
 }
 
 extern "C" int enumgpu_selftest_rcp(uint64_t n_operands, uint64_t seed, uint64_t* n_mismatch, double* first_bad)
 {
     g_err[0] = 0;
     if (!n_mismatch) return fail(ENUMGPU_ERR_ARG, "selftest_rcp: n_mismatch is NULL");
-    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
-    return rcp_selftest_device(n_operands, seed, n_mismatch, first_bad, nullptr);
+    if (const int rc = require_device()) return rc;
+    return rcp_selftest_device(n_operands, seed, n_mismatch, first_bad);
 }
 
 static bool shared_rcp_trusted(int dev)
@@ -1456,7 +1510,7 @@ static bool shared_rcp_trusted(int dev)
     if (t.rcp_state == 0) {
         uint64_t bad = 1;
         double first = 0.0;
-        const int rc = rcp_selftest_device(1ull << 22, 0x5EEDull, &bad, &first, nullptr);
+        const int rc = rcp_selftest_device(1ull << 22, 0x5EEDull, &bad, &first);
         t.rcp_state = (rc == 0 && bad == 0) ? 1 : 2;
         if (t.rcp_state == 2)
             fail(ENUMGPU_OK, "warning: the shared kernel's reciprocal differs from __drcp_rn on device %d (%llu of 2^22 operands, "
@@ -1509,8 +1563,8 @@ extern "C" int enumgpu_create(int32_t device, enumgpu_handle** out)
     g_err[0] = 0;
     if (!out) return fail(ENUMGPU_ERR_ARG, "create: out is NULL");
     *out = nullptr;
-    const int have = enumgpu_device_count();
-    if (have < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
+    int have = 0;
+    if (const int rc = require_device(&have)) return rc;
     int cur = 0;
     cudaGetDevice(&cur);
     if (device < 0) device = cur;
@@ -1574,35 +1628,24 @@ extern "C" int enumgpu_solve_hv(enumgpu_handle* const* hs, int32_t n_handles, co
     Resolved rs;
     int rc = resolve(p, o, &rs, true);
     if (rc) return out->status = rc;
-    const int m = p->m, n = p->n;
-    // pack A (lda -> m), b, c into the pinned staging buffer of handle 0; max|A_ij| in the same pass
+    // the packed problem in the pinned staging buffer of handle 0
     enumgpu_handle* h0 = hs[0];
-    double scale = 0.0;
-    for (int j = 0; j < n; ++j)
-        for (int i = 0; i < m; ++i) {
-            const double v = p->A_colmajor[i + (size_t)j * p->lda];
-            h0->h_in[(size_t)j * m + i] = v;
-            scale = fmax(scale, fabs(v));
-        }
-    memcpy(h0->h_in + (size_t)m * n, p->b, sizeof(double) * m);
-    memcpy(h0->h_in + (size_t)m * n + m, p->c, sizeof(double) * n);
-    const size_t bytes = ((size_t)m * n + m + n) * sizeof(double);
+    const double scale = pack_problem(p, h0->h_in);
+    const size_t bytes = packed_doubles(p) * sizeof(double);
     int cur = 0;
     cudaGetDevice(&cur);
     int32_t launches[ENUMGPU_MAX_DEVICES] = {0};
     auto body = [&]() -> int {
         for (int i = 0; i < n_handles; ++i) {
             enumgpu_handle* h = hs[i];
-            const uint32_t sh_index = rs.shard_index + rs.shard_count * (uint32_t)i, sh_count = rs.shard_count * (uint32_t)n_handles;
+            Resolved rd = rs;
+            rd.shard_index = rs.shard_index + rs.shard_count * (uint32_t)i;
+            rd.shard_count = rs.shard_count * (uint32_t)n_handles;
             CU(cudaSetDevice(h->dev));
             CU(cudaMemcpyAsync(h->d_in, h0->h_in, bytes, cudaMemcpyHostToDevice, h->st));
-            enumgpu_problem dp = *p;
-            dp.lda = m;
-            dp.A_colmajor = h->d_in;
-            dp.b = h->d_in + (size_t)m * n;
-            dp.c = dp.b + m;
+            const enumgpu_problem dp = packed_view(p, h->d_in);
             CU(cudaEventRecord(h->e0, h->st));
-            const int r2 = enqueue_range(&dp, scale, rs, rs.begin, rs.end, sh_index, sh_count, h->st, h->d_part, &launches[i], &h->scratch);
+            const int r2 = enqueue_range(&dp, scale, rd, h->st, h->d_part, &launches[i], &h->scratch);
             if (r2) return r2;
             CU(cudaEventRecord(h->e1, h->st));
             CU(cudaMemcpyAsync(h->h_part, h->d_part, sizeof(enumgpu_partial), cudaMemcpyDeviceToHost, h->st));
@@ -1638,22 +1681,38 @@ extern "C" int enumgpu_solve_h(enumgpu_handle* h, const enumgpu_problem* p, cons
     return enumgpu_solve_hv(&h, 1, p, o, out);
 }
 
-extern "C" int enumgpu_enqueue_h(enumgpu_handle* h, const enumgpu_problem* p_dev, double scale_A, const enumgpu_options* o,
-                                 enumgpu_partial* partial_dev, int32_t* n_launches)
+// enumgpu_enqueue_h (host_ptrs false: p and scale_A as the caller gives them) and enumgpu_enqueue_host_h (host_ptrs
+// true: p is packed into the handle's pinned staging buffer and copied to the device first), on o->stream or the
+// handle's stream.  A failure leaves the handle ready for the next call.
+static int handle_enqueue(const char* who, enumgpu_handle* h, const enumgpu_problem* p, bool host_ptrs, double scale_A,
+                          const enumgpu_options* o, enumgpu_partial* partial_dev, int32_t* n_launches)
 {
     g_err[0] = 0;
     if (!h) return fail(ENUMGPU_ERR_ARG, "handle is NULL");
     Resolved rs;
-    int rc = resolve(p_dev, o, &rs, false);
+    int rc = resolve(p, o, &rs, host_ptrs);
     if (rc) return rc;
     if (!partial_dev) return fail(ENUMGPU_ERR_ARG, "partial_dev is NULL");
     int cur = 0;
     cudaGetDevice(&cur);
-    if (cur != h->dev) return fail(ENUMGPU_ERR_ARG, "enqueue_h: the handle belongs to device %d, the current device is %d", h->dev, cur);
+    if (cur != h->dev) return fail(ENUMGPU_ERR_ARG, "%s: the handle belongs to device %d, the current device is %d", who, h->dev, cur);
     cudaStream_t st = (o && o->stream) ? (cudaStream_t)o->stream : h->st;
-    rc = enqueue_range(p_dev, scale_A, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, partial_dev, n_launches, &h->scratch);
+    enumgpu_problem dp = *p;
+    if (host_ptrs) {
+        scale_A = pack_problem(p, h->h_in);
+        dp = packed_view(p, h->d_in);
+        const cudaError_t e = cudaMemcpyAsync(h->d_in, h->h_in, packed_doubles(p) * sizeof(double), cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) rc = fail(ENUMGPU_ERR_CUDA, "%s: H2D copy failed: %s", who, cudaGetErrorString(e));
+    }
+    if (rc == 0) rc = enqueue_range(&dp, scale_A, rs, st, partial_dev, n_launches, &h->scratch);
     if (rc) { cudaStreamSynchronize(st); handle_recover(h); }
     return rc;
+}
+
+extern "C" int enumgpu_enqueue_h(enumgpu_handle* h, const enumgpu_problem* p_dev, double scale_A, const enumgpu_options* o,
+                                 enumgpu_partial* partial_dev, int32_t* n_launches)
+{
+    return handle_enqueue("enqueue_h", h, p_dev, false, scale_A, o, partial_dev, n_launches);
 }
 
 // enumgpu_enqueue_h for HOST inputs: pack A|b|c into the handle's pinned staging buffer, one H2D copy and the
@@ -1662,38 +1721,7 @@ extern "C" int enumgpu_enqueue_h(enumgpu_handle* h, const enumgpu_problem* p_dev
 extern "C" int enumgpu_enqueue_host_h(enumgpu_handle* h, const enumgpu_problem* p, const enumgpu_options* o,
                                       enumgpu_partial* partial_dev, int32_t* n_launches)
 {
-    g_err[0] = 0;
-    if (!h) return fail(ENUMGPU_ERR_ARG, "handle is NULL");
-    Resolved rs;
-    int rc = resolve(p, o, &rs, true);
-    if (rc) return rc;
-    if (!partial_dev) return fail(ENUMGPU_ERR_ARG, "partial_dev is NULL");
-    int cur = 0;
-    cudaGetDevice(&cur);
-    if (cur != h->dev) return fail(ENUMGPU_ERR_ARG, "enqueue_host_h: the handle belongs to device %d, the current device is %d", h->dev, cur);
-    const int m = p->m, n = p->n;
-    double scale = 0.0;
-    for (int j = 0; j < n; ++j)
-        for (int i = 0; i < m; ++i) {
-            const double v = p->A_colmajor[i + (size_t)j * p->lda];
-            h->h_in[(size_t)j * m + i] = v;
-            scale = fmax(scale, fabs(v));
-        }
-    memcpy(h->h_in + (size_t)m * n, p->b, sizeof(double) * m);
-    memcpy(h->h_in + (size_t)m * n + m, p->c, sizeof(double) * n);
-    cudaStream_t st = (o && o->stream) ? (cudaStream_t)o->stream : h->st;
-    auto body = [&]() -> int {
-        CU(cudaMemcpyAsync(h->d_in, h->h_in, ((size_t)m * n + m + n) * sizeof(double), cudaMemcpyHostToDevice, st));
-        enumgpu_problem dp = *p;
-        dp.lda = m;
-        dp.A_colmajor = h->d_in;
-        dp.b = h->d_in + (size_t)m * n;
-        dp.c = dp.b + m;
-        return enqueue_range(&dp, scale, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, partial_dev, n_launches, &h->scratch);
-    };
-    rc = body();
-    if (rc) { cudaStreamSynchronize(st); handle_recover(h); }
-    return rc;
+    return handle_enqueue("enqueue_host_h", h, p, true, 0.0, o, partial_dev, n_launches);
 }
 
 // merge n partial records (host memory, e.g. the result of an all-gather) into one result struct
@@ -1713,42 +1741,11 @@ extern "C" int enumgpu_solve_device(const enumgpu_problem* p_dev, double scale_A
     memset(out, 0, sizeof *out);
     Resolved rs;
     int rc = resolve(p_dev, o, &rs, false);
+    if (rc == 0) rc = require_device();
     if (rc) return out->status = rc;
-    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
-
-    cudaStream_t st = o ? (cudaStream_t)o->stream : nullptr;
-    bool own_stream = false;
-    if (!st) {
-        if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess)
-            return out->status = fail(ENUMGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(cudaGetLastError()));
-        own_stream = true;
-    }
-    enumgpu_partial h_part;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    int32_t launches = 0;
-    auto body = [&]() -> int {
-        CU(cudaEventCreate(&e0));
-        CU(cudaEventCreate(&e1));
-        StreamBuf b_part;
-        CU(b_part.alloc(sizeof(enumgpu_partial), st));
-        enumgpu_partial* d_part = b_part.as<enumgpu_partial>();
-        CU(cudaEventRecord(e0, st));
-        int r2 = enqueue_range(p_dev, scale_A, rs, rs.begin, rs.end, rs.shard_index, rs.shard_count, st, d_part, &launches);
-        if (r2) return r2;
-        CU(cudaEventRecord(e1, st));
-        CU(cudaMemcpyAsync(&h_part, d_part, sizeof h_part, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, e0, e1));
-        enumgpu_partial_to_result(&h_part, out);
-        out->kernel_ms = ms;
-        out->n_launches = launches;
-        return 0;
-    };
-    rc = body();
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (own_stream) cudaStreamDestroy(st);
+    CallStream cs;
+    rc = cs.open(true, o ? (cudaStream_t)o->stream : nullptr);
+    if (rc == 0) rc = enumerate_timed(p_dev, scale_A, rs, cs, nullptr, nullptr, out);
     if (rc) { out->status = rc; return rc; }
     return out->status;
 }
@@ -1762,9 +1759,9 @@ extern "C" int enumgpu_solve(const enumgpu_problem* p, const enumgpu_options* o,
     memset(out, 0, sizeof *out);
     Resolved rs;
     int rc = resolve(p, o, &rs, true);
+    int have = 0;
+    if (rc == 0) rc = require_device(&have);
     if (rc) return out->status = rc;
-    const int have = enumgpu_device_count();
-    if (have < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
 
     int nd = (o && o->n_devices > 0) ? o->n_devices : 1;
     if (nd > ENUMGPU_MAX_DEVICES) return out->status = fail(ENUMGPU_ERR_ARG, "n_devices=%d above %d", nd, ENUMGPU_MAX_DEVICES);
@@ -1811,11 +1808,9 @@ extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options*
     if (rc) return out->status = rc;
     const int m = p->m, n = p->n, ma = m + 1;
     if (ma > kMaxM) return out->status = fail(ENUMGPU_ERR_ARG, "find_ray: the auxiliary LP needs m+1 = %d rows, above %d", ma, kMaxM);
-    double amax = 0.0, cmax = 0.0;
-    for (int j = 0; j < n; ++j) {
-        cmax = fmax(cmax, fabs(p->c[j]));
-        for (int i = 0; i < m; ++i) amax = fmax(amax, fabs(p->A_colmajor[i + (size_t)j * p->lda]));
-    }
+    const double amax = max_abs_A(p);
+    double cmax = 0.0;
+    for (int j = 0; j < n; ++j) cmax = fmax(cmax, fabs(p->c[j]));
     out->m = ma;
     if (n < ma || cmax == 0.0) {          // no basis of m+1 columns, or no direction can decrease ck.x
         out->key = INFINITY; out->best_rank = UINT64_MAX; out->objective = NAN;
@@ -1842,29 +1837,19 @@ extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options*
 // slabs and the staging of the bases and certificates are sized by the chunk, not by the number of bases.
 constexpr uint32_t kCertifyChunk = 4096;
 struct Certifier {
-    struct OwnedStream {               // declared first: destroyed after the buffers have queued their frees on it
-        cudaStream_t s = nullptr;
-        ~OwnedStream() { if (s) cudaStreamDestroy(s); }
-    } owned;
-    cudaStream_t st = nullptr;
+    CallStream cs;                     // declared first: destroyed after the buffers have queued their frees on it
     DeviceProblem D;
     StreamBuf b_scratch, b_S, b_out;
     double thr = 0.0;
-    int32_t launches = 0;
 
     int init(const enumgpu_problem* p, const Resolved& rs)
     {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        keep_pool_memory(dev);
-        CU(cudaStreamCreateWithFlags(&owned.s, cudaStreamNonBlocking));
-        st = owned.s;
-        const int rc = upload_problem(p, st, &D);
-        if (rc) return rc;
-        thr = rs.rule == ENUMGPU_PIVOT_RELATIVE ? 0.0 : rs.eps_piv * D.scale;
-        CU(b_scratch.alloc(sizeof(double) * certify_slab(p->m, p->n) * kCertifyChunk, st));
-        CU(b_S.alloc(sizeof(int32_t) * p->m * kCertifyChunk, st));
-        CU(b_out.alloc(sizeof(enumgpu_certificate) * kCertifyChunk, st));
+        int rc;
+        if ((rc = cs.open(false)) || (rc = upload_problem(p, cs.st, &D))) return rc;
+        thr = pivot_threshold(rs, D.scale);
+        CU(b_scratch.alloc(sizeof(double) * certify_slab(p->m, p->n) * kCertifyChunk, cs.st));
+        CU(b_S.alloc(sizeof(int32_t) * p->m * kCertifyChunk, cs.st));
+        CU(b_out.alloc(sizeof(enumgpu_certificate) * kCertifyChunk, cs.st));
         return 0;
     }
     // count <= kCertifyChunk bases of m columns each (host); out[i] as the kernel leaves it, n_launches = 1
@@ -1872,25 +1857,18 @@ struct Certifier {
             enumgpu_certificate* out)
     {
         const int m = p->m, n = p->n;
-        CU(cudaMemcpyAsync(b_S.p, bases, sizeof(int32_t) * m * count, cudaMemcpyHostToDevice, st));
-        CU(cudaMemsetAsync(b_out.p, 0, sizeof(enumgpu_certificate) * count, st));
-        k_certify<<<count, kCertifyThreads, 0, st>>>(D.dp.A_colmajor, D.dp.b, D.dp.c, b_S.as<int>(), m, n, p->maximize ? 1 : 0,
-                                                     thr, rs.eps_feas, rs.rule, rs.eps_piv, eps_opt, b_scratch.as<double>(),
-                                                     b_out.as<enumgpu_certificate>());
+        CU(cudaMemcpyAsync(b_S.p, bases, sizeof(int32_t) * m * count, cudaMemcpyHostToDevice, cs.st));
+        CU(cudaMemsetAsync(b_out.p, 0, sizeof(enumgpu_certificate) * count, cs.st));
+        k_certify<<<count, kCertifyThreads, 0, cs.st>>>(D.dp.A_colmajor, D.dp.b, D.dp.c, b_S.as<int>(), m, n, p->maximize ? 1 : 0,
+                                                        thr, rs.eps_feas, rs.rule, rs.eps_piv, eps_opt, b_scratch.as<double>(),
+                                                        b_out.as<enumgpu_certificate>());
         CU(cudaGetLastError());
-        ++launches;
-        CU(cudaMemcpyAsync(out, b_out.p, sizeof(enumgpu_certificate) * count, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        CU(cudaMemcpyAsync(out, b_out.p, sizeof(enumgpu_certificate) * count, cudaMemcpyDeviceToHost, cs.st));
+        CU(cudaStreamSynchronize(cs.st));
         for (uint32_t i = 0; i < count; ++i) out[i].n_launches = 1;
         return 0;
     }
 };
-
-static double resolve_eps_opt(double eps_opt)
-{
-    if (!(eps_opt >= 0)) return 1e-9;                    // negative (or NaN): the default
-    return eps_opt == 0.0 ? 0.0 : eps_opt;               // -0.0 means 0
-}
 
 static int check_bases(const enumgpu_problem* p, const int32_t* bases, uint64_t count, const char* who)
 {
@@ -1904,9 +1882,9 @@ static int check_bases(const enumgpu_problem* p, const int32_t* bases, uint64_t 
 static int certify_one(const enumgpu_problem* p, const Resolved& rs, const int32_t* basis, double eps_opt,
                        enumgpu_certificate* out)
 {
-    if (enumgpu_device_count() < 1) return out->status = fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
     Certifier cf;
-    int rc = cf.init(p, rs);
+    int rc = require_device();
+    if (rc == 0) rc = cf.init(p, rs);
     if (rc == 0) rc = cf.run(p, rs, basis, 1, eps_opt, out);
     if (rc) { out->status = rc; return rc; }
     if (out->basis_class != ENUMGPU_BASIS_FEASIBLE)
@@ -1959,10 +1937,9 @@ extern "C" int enumgpu_certify_bases(const enumgpu_problem* p, const enumgpu_opt
     int rc = resolve(p, &oc, &rs, true);
     if (rc || (rc = check_bases(p, bases, count, "certify_bases"))) return rc;
     if (count == 0) return ENUMGPU_OK;
-    if (enumgpu_device_count() < 1) return fail(ENUMGPU_ERR_CUDA, "no CUDA device available (libenumgpu has no CPU fallback)");
     eps_opt = resolve_eps_opt(eps_opt);
     Certifier cf;
-    if ((rc = cf.init(p, rs))) return rc;
+    if ((rc = require_device()) || (rc = cf.init(p, rs))) return rc;
     for (uint64_t i = 0; i < count; i += kCertifyChunk) {
         const uint32_t k = (uint32_t)std::min<uint64_t>(kCertifyChunk, count - i);
         if ((rc = cf.run(p, rs, bases + i * p->m, k, eps_opt, out + i))) return rc;

@@ -649,6 +649,16 @@ def test_eval_basis_any_size(gpu_lib, oracle):
     assert rep.IsFeasibleBasis() is False
     with pytest.raises(RuntimeError, match="Singular"):
         rep.GetBasicSolution()
+    # eps_feas = eps_piv = -0.0 mean 0 (enumgpu.h): the oracle's answer with both tolerances 0
+    zero = _abi.Options(-0.0, -0.0, 0, 0, 0, 0, None, None, 0, 0, _abi.PIVOT_ABSOLUTE, 0)
+    ps = _abi.Problem(8, 24, 8, 0, A8.ctypes.data, b8.ctypes.data, c8.ctypes.data)
+    for S in ([0, 1, 2, 3, 4, 5, 6, 7], [3, 5, 8, 9, 13, 17, 20, 23], [0, 1, 2, 3, 4, 5, 6, 6]):
+        x, z, cls = (C.c_double * 8)(), C.c_double(), C.c_int32()
+        assert gpu_lib.enumgpu_eval_basis(C.byref(ps), C.byref(zero), (C.c_int32 * 8)(*S), x, C.byref(z), C.byref(cls)) == 0
+        st, xo, zo = oracle.eval_basis(A8, b8, c8, False, S, eps_feas=0.0, eps_piv=0.0)
+        assert cls.value == st
+        if st != _abi.BASIS_SINGULAR:
+            assert list(x) == xo and z.value == zo
 
 
 def test_sharded_enumeration_host_path_single_rank(gpu_lib, oracle):
