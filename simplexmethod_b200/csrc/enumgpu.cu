@@ -884,10 +884,12 @@ static int enqueue_range(const enumgpu_problem* pd, double scale_host, const Res
             const size_t cta = shared_cta_bytes(m, n) + 32, per_warp = (shared_warp_bytes(m, n) + 15) & ~size_t(15);
             int max_smem = 0;
             CU(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-#ifdef ENUMGPU_CHECK
-            max_smem -= 1024;                 // the checked build's static window table
-#endif
-            wpc = (int)(((size_t)max_smem - cta) / per_warp);
+            // the kernel's static shared memory counts against the same maximum as the dynamic window
+            // (without it the window of (m, n) = (10, 64) left too little room and the launch was refused)
+            size_t static_smem = 0;
+            sp.base = prm;                    // m and n select the instantiation
+            CU(dispatch_shared(sp, nullptr, 0, 0, 0, st, &static_smem));
+            wpc = (int)(((size_t)max_smem - cta - static_smem) / per_warp);
             if (wpc > kMaxWarps) wpc = kMaxWarps;
             if (wpc < 1) return fail(ENUMGPU_ERR_ARG, "shared kernel: (m,n)=(%d,%d) does not fit shared memory", m, n);
             smem = cta + per_warp * wpc;

@@ -303,8 +303,8 @@ def problem(A, b, c, mx):
                                    c.ctypes.data)
 
 
-def options(algo=_abi.ALGO_AUTO, rank_begin=0, rank_end=0, devices=None):
-    o = _abi.Options(-1.0, -1.0, rank_begin, rank_end, 0, algo, None, None, 0, 0, 0, 0)
+def options(algo=_abi.ALGO_AUTO, rank_begin=0, rank_end=0, devices=None, eps_feas=-1.0):
+    o = _abi.Options(eps_feas, -1.0, rank_begin, rank_end, 0, algo, None, None, 0, 0, 0, 0)
     if devices:
         o.n_devices, o.devices = len(devices), (C.c_int32 * len(devices))(*devices)
     return o

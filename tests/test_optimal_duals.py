@@ -60,14 +60,14 @@ def twin_many():
     return _TWIN
 
 
-def twin_certify_many(A, b, c, mx, bases, eps_opt=1e-9):
-    """The twin's certificates (absolute pivot rule, default tolerances) at bases [k, m]: (rc [k], [Certificate])."""
+def twin_certify_many(A, b, c, mx, bases, eps_opt=1e-9, eps_feas=1e-9):
+    """The twin's certificates (absolute pivot rule, default eps_piv) at bases [k, m]: (rc [k], [Certificate])."""
     keep, p = problem(A, b, c, mx)
     bases = np.ascontiguousarray(bases, dtype=np.int32).reshape(-1, p.m)
     k = bases.shape[0]
     rc = np.zeros(k, dtype=np.int32)
     out = (_abi.Certificate * k)()
-    twin_many().certify_twin_many(C.byref(p), 1e-9, _abi.PIVOT_ABSOLUTE, 1e-9 * float(np.abs(keep[0]).max()), eps_opt,
+    twin_many().certify_twin_many(C.byref(p), eps_feas, _abi.PIVOT_ABSOLUTE, 1e-9 * float(np.abs(keep[0]).max()), eps_opt,
                                   bases.ctypes.data, k, rc.ctypes.data, out)
     return rc, list(out)
 
@@ -284,22 +284,23 @@ def test_optimum_struct_layout_matches_header(tmp_path):
 
 # --------------------------------------------------------------------------------------------- GPU helpers
 
-def gpu_list_window(L, A, b, c, mx, key_max, algo=_abi.ALGO_AUTO, rank_begin=0, rank_end=0, capacity=1 << 22):
+def gpu_list_window(L, A, b, c, mx, key_max, algo=_abi.ALGO_AUTO, rank_begin=0, rank_end=0, capacity=1 << 22,
+                    eps_feas=-1.0):
     keep, p = problem(A, b, c, mx)
     ranks = np.zeros(capacity, dtype=np.uint64)
     n_listed = C.c_uint64()
     res = _abi.Result()
-    rc = L.enumgpu_list_window(C.byref(p), C.byref(options(algo, rank_begin, rank_end)), key_max,
+    rc = L.enumgpu_list_window(C.byref(p), C.byref(options(algo, rank_begin, rank_end, eps_feas=eps_feas)), key_max,
                                ranks.ctypes.data_as(C.POINTER(C.c_uint64)), capacity, C.byref(n_listed), C.byref(res))
     assert rc in (_abi.OK, _abi.NO_FEASIBLE), sm.last_error()
     return ranks[:n_listed.value].copy(), res
 
 
-def gpu_certify_bases(L, A, b, c, mx, bases):
+def gpu_certify_bases(L, A, b, c, mx, bases, eps_feas=-1.0):
     keep, p = problem(A, b, c, mx)
     arr = np.ascontiguousarray(bases, dtype=np.int32).reshape(-1, p.m)
     out = (_abi.Certificate * arr.shape[0])()
-    rc = L.enumgpu_certify_bases(C.byref(p), C.byref(options()), arr.ctypes.data_as(C.POINTER(C.c_int32)),
+    rc = L.enumgpu_certify_bases(C.byref(p), C.byref(options(eps_feas=eps_feas)), arr.ctypes.data_as(C.POINTER(C.c_int32)),
                                  arr.shape[0], -1.0, out)
     assert rc == _abi.OK, sm.last_error()
     return list(out)

@@ -139,9 +139,11 @@ def all_nan_keys(m, n, seed=0):
 FAMILIES = {"sparse_dyadic": sparse_dyadic, "thirds": thirds, "signed_duplicates": signed_duplicates,
             "network": network, "column_scaled": column_scaled, "huge_rhs": huge_rhs, "huge_cost": huge_cost,
             "tiny_rhs": tiny_rhs}
-# the run-time-n instantiation across m (m >= 12 also runs the odd-column copy of the d loop), n = 64, and the
-# three shapes with kernels compiled for their n
-SHAPES = [(6, 18), (7, 21), (9, 22), (11, 23), (12, 26), (13, 24), (16, 24), (6, 64), (8, 24), (10, 30)]
+# the run-time-n instantiation k_shared<m> for every m from 6 to 16 but 8 and 10 (m >= 12 also runs the odd-column
+# copy of the d loop), n = 64, and the three shapes with kernels compiled for their n; test_wide_shapes.py takes
+# every m to n = 41 .. 64
+SHAPES = [(6, 18), (7, 21), (9, 22), (11, 23), (12, 26), (13, 24), (14, 22), (15, 23), (16, 24), (6, 64), (8, 24),
+          (10, 30)]
 
 
 # --------------------------------------------------------------------------------------------- helpers
