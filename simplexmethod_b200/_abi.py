@@ -110,6 +110,23 @@ class Optimum(C.Structure):
     ]
 
 
+class CostRange(C.Structure):
+    _fields_ = [
+        ("decrease", C.c_double), ("increase", C.c_double),
+        ("decrease_rank", C.c_uint64), ("increase_rank", C.c_uint64),
+        ("decrease_ray", C.c_int32), ("increase_ray", C.c_int32),
+    ]
+
+
+class Ranging(C.Structure):
+    _fields_ = [
+        ("status", C.c_int32), ("n", C.c_int32), ("n_launches", C.c_int32), ("reserved_", C.c_int32),
+        ("n_vertex_bases", C.c_uint64), ("n_ray_bases", C.c_uint64),
+        ("kernel_ms", C.c_double),
+        ("range", CostRange * MAX_N),
+    ]
+
+
 # every symbol include/enumgpu.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "enumgpu_version": (C.c_int, []),
@@ -155,6 +172,8 @@ SYMBOLS = {
                                            C.c_uint64, C.POINTER(Optimum)]),
     "enumgpu_solve_objectives": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.c_int32, C.POINTER(C.c_double),
                                             C.c_int32, C.c_uint64, C.POINTER(Result)]),
+    "enumgpu_cost_ranges": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result), C.c_double, C.c_uint64,
+                                       C.POINTER(Ranging)]),
 }
 
 MAX_OBJECTIVES = 1 << 20

@@ -138,6 +138,15 @@ public:
     const std::vector<int>& certificateBasis() const { certificate(); return cert_basis_; }
     int certificateSource() const { certificate(); return cert_source_; }
 
+    // Cost ranging of the optimum of the last solve() (enumgpu_cost_ranges, current device): for every column j, the
+    // allowable decrease and increase of c_j over which the optimal vertex stays optimal, exact at degenerate
+    // vertices, with the basis or ray that takes over at each end.  Throws std::runtime_error("objective is unbounded")
+    // on an unbounded LP.  eps_opt < 0: 1e-9; max_list = 0: 2^26 ranks held on the device.
+    const enumgpu_ranging& costRanges(double eps_opt = -1.0, uint64_t max_list = 0)
+    {
+        return rangesWith(&enumgpu_cost_ranges, eps_opt, max_list);
+    }
+
 private:
     void need() const { if (!solved_) throw std::logic_error("EnumerationSolver: solve() has not been called"); }
     using CertifyFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const int32_t*, double, enumgpu_certificate*);
@@ -163,6 +172,20 @@ private:
         if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
         certified_ = true;
         return cert_;
+    }
+    using RangesFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const enumgpu_result*, double, uint64_t,
+                             enumgpu_ranging*);
+    const enumgpu_ranging& rangesWith(RangesFn fn, double eps_opt, uint64_t max_list)
+    {
+        need();
+        if (res_.status != ENUMGPU_OK) throw std::runtime_error("the problem has no feasible basic solution");
+        const enumgpu_problem p = problemStruct();
+        const enumgpu_options o = options();
+        const int rc = fn(&p, &o, &res_, eps_opt, max_list, &ranging_);
+        if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
+        if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
+        if (ranging_.status == ENUMGPU_CERT_UNBOUNDED) throw std::runtime_error("objective is unbounded");
+        return ranging_;
     }
     static uint64_t binomial(int n, int k)          // C(n, k) for n <= 64, k <= 16: exact in 64 bits
     {
@@ -224,6 +247,7 @@ private:
     enumgpu_result res_{};
     std::vector<enumgpu_result> obj_res_;      // solveObjectives(), one per cost vector
     enumgpu_certificate cert_{};
+    enumgpu_ranging ranging_{};
     std::vector<int> cert_basis_;
     int cert_source_ = ENUMGPU_OPT_WINNER;
     bool solved_ = false, certified_ = false;

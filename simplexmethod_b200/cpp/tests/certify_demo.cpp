@@ -1,10 +1,12 @@
 // certify_demo.cpp — the certificate of the enumerated optimum through the C++ adapter:
 //   SymmetricalParser::ParseFromFile -> Symmetrical::ToCanonical -> EnumerationSolver::solve() -> certify()
-// usage: certify_demo <symmetric LP file> [--optimal-duals]   prints one machine-readable line per fact: the optimum,
+// usage: certify_demo [--ranges] <symmetric LP file> [--optimal-duals]   prints one machine-readable line per fact: the optimum,
 //        the verdict (ENUMGPU_CERT_*), the entering column of an edge ray, the duals, the reduced costs, the ray, the
 //        counters of the auxiliary enumeration, and whether a solver with setCheckUnbounded(true) reports "objective is
 //        unbounded".  --optimal-duals: both solvers use setOptimalDuals(true), and two more lines give the basis the
 //        certificate belongs to (cert_basis) and where it came from (source, ENUMGPU_OPT_*).
+//        --ranges: the cost ranging table instead (costRanges()): "ranging <status> <vertex bases> <ray bases>", then
+//        one line per canonical column, "range j decrease increase decrease_rank increase_rank decrease_ray increase_ray".
 #include <cstdio>
 #include <cstring>
 #include <exception>
@@ -13,11 +15,36 @@
 #include "EnumerationSolver.h"
 #include "SymmetricalParser.h"
 
+static int print_ranges(const Canonical& can)
+{
+    EnumerationSolver solver(can);
+    solver.solve();
+    const enumgpu_ranging& r = solver.costRanges();
+    std::printf("ranging %d %llu %llu\n", r.status, (unsigned long long)r.n_vertex_bases, (unsigned long long)r.n_ray_bases);
+    for (int j = 0; j < r.n; ++j) {
+        const enumgpu_cost_range& v = r.range[j];
+        std::printf("range %d %.17g %.17g %llu %llu %d %d\n", j, v.decrease, v.increase, (unsigned long long)v.decrease_rank,
+                    (unsigned long long)v.increase_rank, v.decrease_ray, v.increase_ray);
+    }
+    return 0;
+}
+
 int main(int argc, char** argv)
 {
+    if (argc == 3 && !std::strcmp(argv[1], "--ranges")) {
+        SymmetricalParser parser;
+        auto sym = parser.ParseFromFile(argv[2]);
+        if (!sym) { std::fprintf(stderr, "parse error: %s\n", parser.GetLastError().c_str()); return 3; }
+        try {
+            return print_ranges(*sym->ToCanonical());
+        } catch (const std::exception& e) {
+            std::fprintf(stderr, "error: %s\n", e.what());
+            return 1;
+        }
+    }
     const bool optimal_duals = argc == 3 && !std::strcmp(argv[2], "--optimal-duals");
     if (argc < 2 || (argc > 2 && !optimal_duals)) {
-        std::fprintf(stderr, "usage: %s <symmetric LP file> [--optimal-duals]\n", argv[0]);
+        std::fprintf(stderr, "usage: %s [--ranges] <symmetric LP file> [--optimal-duals]\n", argv[0]);
         return 2;
     }
     SymmetricalParser parser;

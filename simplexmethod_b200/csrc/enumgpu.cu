@@ -20,6 +20,7 @@
 #include "k_independent.cuh"
 #include "k_shared.cuh"
 #include "k_objectives.cuh"
+#include "k_ranging.cuh"
 
 using namespace enumgpu;
 
@@ -1257,19 +1258,42 @@ struct ObjPass {
     cudaStream_t st;
 };
 
+// S and x_B of `count` listed ranks of the device problem dp into the chunk buffers S, x ([M][count]): 1 launch
+template <int M>
+static cudaError_t obj_values(const enumgpu_problem& dp, const uint64_t* binom, const uint64_t* ranks, uint32_t count,
+                              uint8_t* S, double* x, cudaStream_t st)
+{
+    const int n = dp.n;
+    const unsigned blocks = (count + kObjThreads - 1) / kObjThreads;
+    if constexpr (M <= 12) {
+        const size_t smem = (size_t)(n * M + M + n) * sizeof(double) + sizeof(uint64_t) * kBinomRows * kBinomCols;
+        k_obj_values<M><<<blocks, kObjThreads, smem, st>>>(dp.A_colmajor, dp.b, binom, n, ranks, count, S, x);
+    } else {
+        k_obj_values_generic<<<blocks, kObjThreads, 0, st>>>(dp.A_colmajor, dp.b, binom, M, n, ranks, count, S, x);
+    }
+    return cudaGetLastError();
+}
+
+static cudaError_t dispatch_obj_values(const enumgpu_problem& dp, const uint64_t* binom, const uint64_t* ranks,
+                                       uint32_t count, uint8_t* S, double* x, cudaStream_t st)
+{
+    switch (dp.m) {
+#define ENUMGPU_CASE(M_) case M_: return obj_values<M_>(dp, binom, ranks, count, S, x, st);
+        ENUMGPU_CASE(1) ENUMGPU_CASE(2) ENUMGPU_CASE(3) ENUMGPU_CASE(4)
+        ENUMGPU_CASE(5) ENUMGPU_CASE(6) ENUMGPU_CASE(7) ENUMGPU_CASE(8)
+        ENUMGPU_CASE(9) ENUMGPU_CASE(10) ENUMGPU_CASE(11) ENUMGPU_CASE(12)
+        ENUMGPU_CASE(13) ENUMGPU_CASE(14) ENUMGPU_CASE(15) ENUMGPU_CASE(16)
+#undef ENUMGPU_CASE
+    }
+    return cudaErrorInvalidValue;
+}
+
 // x_B of `count` listed ranks, then their keys under every cost vector: 2 launches
 template <int M>
 static cudaError_t objectives_chunk(const ObjPass& a, const uint64_t* ranks, uint32_t count, int first)
 {
     const int n = a.dp.n;
-    const unsigned blocks = (count + kObjThreads - 1) / kObjThreads;
-    if constexpr (M <= 12) {
-        const size_t smem = (size_t)(n * M + M + n) * sizeof(double) + sizeof(uint64_t) * kBinomRows * kBinomCols;
-        k_obj_values<M><<<blocks, kObjThreads, smem, a.st>>>(a.dp.A_colmajor, a.dp.b, a.binom, n, ranks, count, a.S, a.x);
-    } else {
-        k_obj_values_generic<<<blocks, kObjThreads, 0, a.st>>>(a.dp.A_colmajor, a.dp.b, a.binom, M, n, ranks, count, a.S, a.x);
-    }
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = obj_values<M>(a.dp, a.binom, ranks, count, a.S, a.x, a.st);
     if (e != cudaSuccess) return e;
     const size_t smem = (size_t)M * kObjTile * (sizeof(double) + 1) + kObjTile * sizeof(uint64_t) + (size_t)n * a.W * sizeof(double);
     e = cudaFuncSetAttribute(k_objectives<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1292,22 +1316,89 @@ static cudaError_t dispatch_objectives(const ObjPass& a, const uint64_t* ranks, 
     return cudaErrorInvalidValue;
 }
 
+// The listing of every feasible basis of a rank range for the entries that consume them all (DESIGN.md §3.2, §3.3).
+// init() sizes the device list: max_list ranks (0 selects 2^26), never more than the largest range has.  run() lists
+// the feasible ranks of rs's range of the device problem D (key bound +inf) and hands each listing to
+// consume(record of the listed range, device ranks, count).  With more feasible bases than the list holds, the range
+// is cut into contiguous sub-ranges of about cap / 2 expected feasible bases each, and one that still overflows is
+// halved; the sub-ranges are consumed in ascending order.  Disjoint ranges merge exactly (enumgpu_merge_partial).
+struct FeasibleLists {
+    StreamBuf b_list, b_count, b_part;
+    uint64_t cap = 0;
+
+    int init(uint64_t max_list, uint64_t max_span, cudaStream_t st)
+    {
+        if (max_list == 0) max_list = 1ull << 26;
+        cap = std::max<uint64_t>(1, std::min(max_list, max_span));
+        CU(b_list.alloc(cap * sizeof(uint64_t), st));
+        CU(b_count.alloc(sizeof(unsigned long long), st));
+        CU(b_part.alloc(sizeof(enumgpu_partial), st));
+        return 0;
+    }
+
+    template <class Consume>
+    int run(const DeviceProblem& D, const Resolved& rs, cudaStream_t st, int32_t* launches, Consume&& consume)
+    {
+        const uint64_t span = rs.end - rs.begin, cap_r = std::max<uint64_t>(1, std::min(cap, span));
+        const Listing listing{b_count.as<unsigned long long>(), b_list.as<uint64_t>(), cap_r, INFINITY};
+        // the feasible ranks of [lo, hi) into b_list (all of them if *count <= cap_r) and the range's record
+        auto list = [&](uint64_t lo, uint64_t hi, enumgpu_partial* lp, uint64_t* count) -> int {
+            CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
+            Resolved sub = rs;
+            sub.begin = lo; sub.end = hi;
+            int32_t nl = 0;
+            const int r3 = enqueue_range(&D.dp, D.scale, sub, st, b_part.as<enumgpu_partial>(), &nl, nullptr, &listing);
+            if (r3) return r3;
+            *launches += nl;
+            unsigned long long h = 0;
+            CU(cudaMemcpyAsync(lp, b_part.p, sizeof *lp, cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(&h, b_count.p, sizeof h, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            *count = h;
+            return 0;
+        };
+        const uint64_t* ranks = b_list.as<uint64_t>();
+        enumgpu_partial lp;
+        uint64_t count = 0;
+        int rc;
+        if ((rc = list(rs.begin, rs.end, &lp, &count))) return rc;
+        if (count <= cap_r) return consume(lp, ranks, count);
+        const uint64_t per = std::max<uint64_t>(1, cap_r / 2), parts = std::min(span, (count + per - 1) / per);
+        std::vector<std::pair<uint64_t, uint64_t>> todo;            // a stack: ascending ranges from its back
+        for (uint64_t i = parts; i-- > 0;)
+            todo.emplace_back(rs.begin + (uint64_t)((unsigned __int128)span * i / parts),
+                              rs.begin + (uint64_t)((unsigned __int128)span * (i + 1) / parts));
+        while (!todo.empty()) {
+            const auto [lo, hi] = todo.back();
+            todo.pop_back();
+            if ((rc = list(lo, hi, &lp, &count))) return rc;
+            if (count <= cap_r) {
+                if ((rc = consume(lp, ranks, count))) return rc;
+                continue;
+            }
+            const uint64_t mid = lo + (hi - lo) / 2;                 // a single rank never overflows: cap_r >= 1
+            todo.emplace_back(mid, hi);
+            todo.emplace_back(lo, mid);
+        }
+        return 0;
+    }
+};
+
 // The device part of enumgpu_solve_objectives for q (c = column 0 of C) and the resolved options: out[0, k).
 static int solve_objectives_device(const enumgpu_problem* q, const Resolved& rs, int32_t k, const double* C, int32_t ldc,
                                    uint64_t max_list, enumgpu_result* out)
 {
     const int m = q->m, n = q->n;
-    if (max_list == 0) max_list = 1ull << 26;
-    // the list never holds more than the range has ranks
-    const uint64_t span = rs.end - rs.begin, cap = std::max<uint64_t>(1, std::min(max_list, span));
-    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, cap);
-
     CallStream cs;
     DeviceProblem D;
-    StreamBuf b_C, b_list, b_count, b_part, b_S, b_x, b_best, b_rec;
+    FeasibleLists fl;
+    StreamBuf b_C, b_S, b_x, b_best, b_rec;
     ObjPass a;
     int rc;
     if ((rc = cs.open(true)) || (rc = upload_problem(q, cs.st, &D)) || (rc = device_binom(cs.dev, &a.binom))) return rc;
+    // the list never holds more than the range has ranks
+    if ((rc = fl.init(max_list, rs.end - rs.begin, cs.st))) return rc;
+    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, fl.cap);
     const cudaStream_t st = cs.st;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cs.dev);
@@ -1324,9 +1415,6 @@ static int solve_objectives_device(const enumgpu_problem* q, const Resolved& rs,
     a.grid = dim3(slices, tiles);
     a.st = st;
     CU(b_C.alloc(hC.size() * sizeof(double), st));
-    CU(b_list.alloc(cap * sizeof(uint64_t), st));
-    CU(b_count.alloc(sizeof(unsigned long long), st));
-    CU(b_part.alloc(sizeof(enumgpu_partial), st));
     CU(b_S.alloc((size_t)chunk * m, st));
     CU(b_x.alloc((size_t)chunk * m * sizeof(double), st));
     CU(b_best.alloc((size_t)slices * k * sizeof(Best), st));
@@ -1335,28 +1423,11 @@ static int solve_objectives_device(const enumgpu_problem* q, const Resolved& rs,
     a.C = b_C.as<double>(); a.S = b_S.as<uint8_t>(); a.x = b_x.as<double>(); a.best = b_best.as<Best>();
     CU(cudaEventRecord(cs.e0, st));
 
-    // the feasible ranks of [lo, hi) into b_list (all of them if *count <= cap) and the range's record
-    const Listing listing{b_count.as<unsigned long long>(), b_list.as<uint64_t>(), cap, INFINITY};
-    auto list = [&](uint64_t lo, uint64_t hi, enumgpu_partial* lp, uint64_t* count) -> int {
-        CU(cudaMemsetAsync(b_count.p, 0, sizeof(unsigned long long), st));
-        Resolved sub = rs;
-        sub.begin = lo; sub.end = hi;
-        int32_t nl = 0;
-        const int r3 = enqueue_range(&D.dp, D.scale, sub, st, b_part.as<enumgpu_partial>(), &nl, nullptr, &listing);
-        if (r3) return r3;
-        launches += nl;
-        unsigned long long h = 0;
-        CU(cudaMemcpyAsync(lp, b_part.p, sizeof *lp, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(&h, b_count.p, sizeof h, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        *count = h;
-        return 0;
-    };
     // every objective's best over the listed ranks, merged into acc with the range's counters
     bool have = false;
-    auto absorb = [&](const enumgpu_partial& lp, uint64_t count) -> int {
+    auto absorb = [&](const enumgpu_partial& lp, const uint64_t* ranks, uint64_t count) -> int {
         for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
-            CU(dispatch_objectives(a, b_list.as<uint64_t>() + c0, (uint32_t)std::min<uint64_t>(chunk, count - c0), c0 == 0));
+            CU(dispatch_objectives(a, ranks + c0, (uint32_t)std::min<uint64_t>(chunk, count - c0), c0 == 0));
             launches += 2;
         }
         k_obj_finish<<<(unsigned)((k + kObjThreads - 1) / kObjThreads), kObjThreads, 0, st>>>(
@@ -1375,32 +1446,7 @@ static int solve_objectives_device(const enumgpu_problem* q, const Resolved& rs,
         have = true;
         return 0;
     };
-    enumgpu_partial lp;
-    uint64_t count = 0;
-    if ((rc = list(rs.begin, rs.end, &lp, &count))) return rc;
-    if (count <= cap) {
-        if ((rc = absorb(lp, count))) return rc;
-    } else {
-        // more feasible bases than the list holds: contiguous sub-ranges of about cap / 2 expected feasible bases
-        // each, and one that still overflows is halved.  Disjoint ranges merge exactly (enumgpu_merge_partial).
-        const uint64_t per = std::max<uint64_t>(1, cap / 2), parts = std::min(span, (count + per - 1) / per);
-        std::vector<std::pair<uint64_t, uint64_t>> todo;            // a stack: ascending ranges from its back
-        for (uint64_t i = parts; i-- > 0;)
-            todo.emplace_back(rs.begin + (uint64_t)((unsigned __int128)span * i / parts),
-                              rs.begin + (uint64_t)((unsigned __int128)span * (i + 1) / parts));
-        while (!todo.empty()) {
-            const auto [lo, hi] = todo.back();
-            todo.pop_back();
-            if ((rc = list(lo, hi, &lp, &count))) return rc;
-            if (count <= cap) {
-                if ((rc = absorb(lp, count))) return rc;
-                continue;
-            }
-            const uint64_t mid = lo + (hi - lo) / 2;                 // a single rank never overflows: cap >= 1
-            todo.emplace_back(mid, hi);
-            todo.emplace_back(lo, mid);
-        }
-    }
+    if ((rc = fl.run(D, rs, st, &launches, absorb))) return rc;
     CU(cudaEventRecord(cs.e1, st));
     CU(cudaStreamSynchronize(st));
     float ms = 0.f;
@@ -1796,9 +1842,39 @@ static enumgpu_options whole_space_options(const enumgpu_options* o)
     return oc;
 }
 
-// The auxiliary LP [A; s*ck'] d = (0, ..., 0, -1), cost 0, minimise: its feasible bases are the extreme rays of
-// {d >= 0, A d = 0} with ck.d < 0.  s = 2^e, the largest power of two with s*max|ck_j| <= max|A_ij|, keeps
-// max|A'_ij| = max|A_ij| and with it the pivot threshold.
+// The auxiliary LP of the ray enumerations: [A; s*row'] d = (0, ..., 0, rhs), cost 0, minimise; the caller sets rhs
+// (b[m]).  s = 2^e, the largest power of two with s*max|row_j| <= max|A_ij|, keeps max|A'_ij| = max|A_ij| and with it
+// the pivot threshold.  max|row_j| > 0.  ENUMGPU_ERR_RANGE when max|A_ij| = 0 or scaling by s would lose bits of a row_j.
+struct AuxLP {
+    std::vector<double> A, b, c;
+    enumgpu_problem p;
+    double s;
+};
+static int build_aux_lp(const enumgpu_problem* p, const double* row, const char* who, AuxLP* out)
+{
+    const int m = p->m, n = p->n, ma = m + 1;
+    const double amax = max_abs_A(p);
+    double rmax = 0.0;
+    for (int j = 0; j < n; ++j) rmax = fmax(rmax, fabs(row[j]));
+    if (amax == 0.0) return fail(ENUMGPU_ERR_RANGE, "%s: A = 0 leaves no scale for the auxiliary row", who);
+    int ea = 0, er = 0;
+    const double fa = frexp(amax, &ea), fr = frexp(rmax, &er);
+    const int e = ea - er - (fr > fa ? 1 : 0);
+    out->A.assign((size_t)ma * n, 0.0);
+    out->b.assign(ma, 0.0);
+    out->c.assign(n, 0.0);
+    for (int j = 0; j < n; ++j) {
+        for (int i = 0; i < m; ++i) out->A[(size_t)j * ma + i] = p->A_colmajor[i + (size_t)j * p->lda];
+        const double v = ldexp(row[j], e);
+        if (ldexp(v, -e) != row[j]) return fail(ENUMGPU_ERR_RANGE, "%s: row[%d] * 2^%d is not exact", who, j, e);
+        out->A[(size_t)j * ma + m] = v;
+    }
+    out->s = ldexp(1.0, e);
+    out->p = enumgpu_problem{ma, n, ma, 0, out->A.data(), out->b.data(), out->c.data()};
+    return 0;
+}
+
+// The auxiliary LP with row ck and rhs -1: its feasible bases are the extreme rays of {d >= 0, A d = 0} with ck.d < 0.
 extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options* o, enumgpu_result* out)
 {
     g_err[0] = 0;
@@ -1810,29 +1886,21 @@ extern "C" int enumgpu_find_ray(const enumgpu_problem* p, const enumgpu_options*
     if (rc) return out->status = rc;
     const int m = p->m, n = p->n, ma = m + 1;
     if (ma > kMaxM) return out->status = fail(ENUMGPU_ERR_ARG, "find_ray: the auxiliary LP needs m+1 = %d rows, above %d", ma, kMaxM);
-    const double amax = max_abs_A(p);
+    std::vector<double> ck(n);
     double cmax = 0.0;
-    for (int j = 0; j < n; ++j) cmax = fmax(cmax, fabs(p->c[j]));
+    for (int j = 0; j < n; ++j) {
+        ck[j] = p->maximize ? -p->c[j] : p->c[j];
+        cmax = fmax(cmax, fabs(p->c[j]));
+    }
     out->m = ma;
     if (n < ma || cmax == 0.0) {          // no basis of m+1 columns, or no direction can decrease ck.x
         out->key = INFINITY; out->best_rank = UINT64_MAX; out->objective = NAN;
         return out->status = ENUMGPU_NO_FEASIBLE;
     }
-    if (amax == 0.0) return out->status = fail(ENUMGPU_ERR_RANGE, "find_ray: A = 0 leaves no scale for the cost row");
-    int ea = 0, ec = 0;
-    const double fa = frexp(amax, &ea), fc = frexp(cmax, &ec);
-    const int e = ea - ec - (fc > fa ? 1 : 0);
-    std::vector<double> Aa((size_t)ma * n), ba(ma, 0.0), ca(n, 0.0);
-    for (int j = 0; j < n; ++j) {
-        for (int i = 0; i < m; ++i) Aa[(size_t)j * ma + i] = p->A_colmajor[i + (size_t)j * p->lda];
-        const double ck = p->maximize ? -p->c[j] : p->c[j];
-        const double v = ldexp(ck, e);
-        if (ldexp(v, -e) != ck) return out->status = fail(ENUMGPU_ERR_RANGE, "find_ray: c[%d] * 2^%d is not exact", j, e);
-        Aa[(size_t)j * ma + m] = v;
-    }
-    ba[m] = -1.0;
-    const enumgpu_problem aux{ma, n, ma, 0, Aa.data(), ba.data(), ca.data()};
-    return enumgpu_solve(&aux, o, out);
+    AuxLP aux;
+    if ((rc = build_aux_lp(p, ck.data(), "find_ray", &aux))) return out->status = rc;
+    aux.b[m] = -1.0;
+    return enumgpu_solve(&aux.p, o, out);
 }
 
 // k_certify on a list of bases, kCertifyChunk blocks per launch at most: the device copy of the LP, the scratch
@@ -2015,6 +2083,137 @@ extern "C" int enumgpu_certify_optimum(const enumgpu_problem* p, const enumgpu_o
     rc = ray_fallback(p, &oc, &out->cert);
     out->n_launches += out->cert.n_launches - before;
     return rc;
+}
+
+// ------------------------------------------------------------------ cost ranging (DESIGN.md §3.3)
+
+// The device part of enumgpu_cost_ranges: both listings, the ranging kernels over each listed chunk, the finish.
+// aux: the ray LP, or NULL where m + 1 rows do not fit or n = m.
+static int cost_ranges_device(const enumgpu_problem* p, const Resolved& rs, const AuxLP* aux, const Resolved& rsa,
+                              const enumgpu_result* opt, double eps_opt, uint64_t max_list, enumgpu_ranging* out)
+{
+    const int m = p->m, n = p->n, rows = aux ? m + 1 : m;
+    CallStream cs;
+    DeviceProblem D, Da;
+    FeasibleLists fl;
+    StreamBuf b_S, b_x, b_vec, b_Sstar, b_best, b_flags, b_out;
+    const uint64_t* binom = nullptr;
+    int rc;
+    if ((rc = cs.open(true)) || (rc = upload_problem(p, cs.st, &D)) || (rc = device_binom(cs.dev, &binom))) return rc;
+    if (aux && (rc = upload_problem(&aux->p, cs.st, &Da))) return rc;
+    const cudaStream_t st = cs.st;
+    if ((rc = fl.init(max_list, std::max(rs.total, aux ? rsa.total : 0), st))) return rc;
+    const uint32_t chunk = (uint32_t)std::min<uint64_t>(kObjChunk, fl.cap);
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cs.dev);
+    const unsigned slices = (unsigned)(4 * sms);
+    // c | ck | x* | eps_opt * max(1, |x*_j|)
+    std::vector<double> vec((size_t)4 * n, 0.0);
+    for (int j = 0; j < n; ++j) {
+        vec[j] = p->c[j];
+        vec[n + j] = p->maximize ? -p->c[j] : p->c[j];
+    }
+    for (int i = 0; i < m; ++i) vec[2 * n + opt->basis[i]] = opt->x_B[i];
+    for (int j = 0; j < n; ++j) vec[3 * n + j] = eps_opt * fmax(1.0, fabs(vec[2 * n + j]));
+    const double key_star = opt->key, tau_k = eps_opt * fmax(1.0, fabs(key_star));
+    CU(b_S.alloc((size_t)chunk * rows, st));
+    CU(b_x.alloc((size_t)chunk * rows * sizeof(double), st));
+    CU(b_vec.alloc(vec.size() * sizeof(double), st));
+    CU(b_Sstar.alloc(sizeof(int32_t) * m, st));
+    CU(b_best.alloc((size_t)slices * 3 * n * sizeof(Best), st));
+    CU(b_flags.alloc(2 * sizeof(int), st));
+    CU(b_out.alloc((size_t)n * sizeof(enumgpu_cost_range), st));
+    CU(cudaMemcpyAsync(b_vec.p, vec.data(), vec.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(b_Sstar.p, opt->basis, sizeof(int32_t) * m, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(b_flags.p, 0, 2 * sizeof(int), st));
+    const double* d_vec = b_vec.as<double>();
+    int32_t launches = 0;
+    CU(cudaEventRecord(cs.e0, st));
+
+    // the candidates of every listed basis of the family `ray` (problem *P) folded into the slices' minima
+    bool have[2] = {false, false};
+    int ray = 0;
+    const DeviceProblem* P = &D;
+    uint64_t* n_bases = &out->n_vertex_bases;
+    auto absorb = [&](const enumgpu_partial& lp, const uint64_t* ranks, uint64_t count) -> int {
+        *n_bases += lp.n_feasible;
+        for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
+            const uint32_t k = (uint32_t)std::min<uint64_t>(chunk, count - c0);
+            CU(dispatch_obj_values(P->dp, binom, ranks + c0, k, b_S.as<uint8_t>(), b_x.as<double>(), st));
+            k_ranging<<<slices, kRangeThreads, 0, st>>>(b_S.as<uint8_t>(), b_x.as<double>(), ranks + c0, k, P->dp.m, n, ray,
+                                                       p->maximize ? 1 : 0, d_vec + (ray ? n : 0), d_vec + 2 * n, d_vec + 3 * n,
+                                                       b_Sstar.as<int32_t>(), m, key_star, tau_k, eps_opt, have[ray] ? 0 : 1,
+                                                       b_best.as<Best>(), b_flags.as<int>());
+            CU(cudaGetLastError());
+            launches += 2;
+            have[ray] = true;
+        }
+        return 0;
+    };
+    if ((rc = fl.run(D, rs, st, &launches, absorb))) return rc;
+    if (aux) {
+        ray = 1; P = &Da; n_bases = &out->n_ray_bases;
+        if ((rc = fl.run(Da, rsa, st, &launches, absorb))) return rc;
+    }
+    k_ranging_finish<<<(unsigned)((n + kRangeThreads - 1) / kRangeThreads), kRangeThreads, 0, st>>>(
+        b_best.as<Best>(), have[0] ? (int)slices : 0, have[1] ? (int)slices : 0, n, p->maximize ? 1 : 0,
+        b_out.as<enumgpu_cost_range>());
+    CU(cudaGetLastError());
+    ++launches;
+    CU(cudaEventRecord(cs.e1, st));
+    int flags[2] = {0, 0};
+    CU(cudaMemcpyAsync(out->range, b_out.p, (size_t)n * sizeof(enumgpu_cost_range), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(flags, b_flags.p, sizeof flags, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    out->kernel_ms = ms;
+    out->n_launches = launches;
+    if (flags[0]) return fail(ENUMGPU_ERR_ARG, "cost_ranges: a feasible basis has a key below opt->key (opt came from other options)");
+    if (flags[1]) {
+        out->status = ENUMGPU_CERT_UNBOUNDED;
+        for (int j = 0; j < n; ++j)
+            out->range[j] = enumgpu_cost_range{NAN, NAN, UINT64_MAX, UINT64_MAX, 0, 0};
+    } else {
+        out->status = (m + 1 > kMaxM && n > m) ? ENUMGPU_CERT_UNDECIDED : ENUMGPU_CERT_OPTIMAL;
+    }
+    return ENUMGPU_OK;
+}
+
+extern "C" int enumgpu_cost_ranges(const enumgpu_problem* p, const enumgpu_options* o, const enumgpu_result* opt,
+                                   double eps_opt, uint64_t max_list, enumgpu_ranging* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "cost_ranges: out is NULL");
+    memset(out, 0, sizeof *out);
+    if (o && (o->rank_begin != 0 || o->rank_end != 0))
+        return out->status = fail(ENUMGPU_ERR_ARG, "cost_ranges: a rank range is not supported (the ranges are a statement about the whole space)");
+    if (o && (o->shard_index != 0 || o->shard_count != 0))
+        return out->status = fail(ENUMGPU_ERR_ARG, "cost_ranges: shards are not supported");
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs, rsa{};
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc) return out->status = rc;
+    const int m = p->m, n = p->n;
+    out->n = n;
+    if (!opt || opt->status != ENUMGPU_OK || opt->m != m || opt->n_bases != rs.total)
+        return out->status = fail(ENUMGPU_ERR_ARG, "cost_ranges: opt is not the whole-range optimum of this LP (status OK, m = %d, n_bases = C(%d, %d))", m, n, m);
+    int32_t S[kMaxM];
+    if (opt->best_rank >= rs.total || enumgpu_unrank(n, m, opt->best_rank, S) != 0 || memcmp(S, opt->basis, sizeof(int32_t) * m))
+        return out->status = fail(ENUMGPU_ERR_ARG, "cost_ranges: opt->basis is not unrank(opt->best_rank)");
+    eps_opt = resolve_eps_opt(eps_opt);
+    // the rays: the feasible bases of [A; s*1'] d = (0, ..., 0, s), normalised to 1'd = 1
+    AuxLP aux;
+    const bool rays = m + 1 <= kMaxM && n > m;
+    if (rays) {
+        const std::vector<double> ones(n, 1.0);
+        if ((rc = build_aux_lp(p, ones.data(), "cost_ranges", &aux))) return out->status = rc;
+        aux.b[m] = aux.s;
+        if ((rc = resolve(&aux.p, &oc, &rsa, true))) return out->status = rc;
+    }
+    if ((rc = require_device()) || (rc = cost_ranges_device(p, rs, rays ? &aux : nullptr, rsa, opt, eps_opt, max_list, out)))
+        return out->status = rc;
+    return ENUMGPU_OK;
 }
 
 #ifdef ENUMGPU_TRACE

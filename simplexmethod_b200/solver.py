@@ -14,7 +14,7 @@ include/enumgpu.h; this module only marshals buffers.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence
+from typing import NamedTuple, Optional, Sequence
 
 import numpy as np
 
@@ -155,6 +155,24 @@ def _check(rc: int):
         raise EnumGpuError(last_error())
     if rc in (_abi.ERR_ARG, _abi.ERR_RANGE, _abi.ERR_NONFINITE):
         raise ValueError(last_error())
+
+
+class CostRanges(NamedTuple):
+    """Cost ranging of EnumerationSolver.costRanges(): for each canonical column j, c_j can fall by decrease[j] or
+    rise by increase[j] (np.inf: without limit) and the optimal vertex stays optimal.  *_rank[j] is the basis that
+    takes over at that end (UINT64_MAX: none); where *_ray[j] is True it is an extreme ray, a rank among the
+    C(n, m+1) bases of the auxiliary LP.  status is CERT_OPTIMAL (exact) or CERT_UNDECIDED (m = 16: no rays
+    enumerated; the ranges on the side rays can limit are upper bounds)."""
+    status: int
+    decrease: np.ndarray
+    increase: np.ndarray
+    decrease_rank: np.ndarray
+    increase_rank: np.ndarray
+    decrease_ray: np.ndarray
+    increase_ray: np.ndarray
+    n_vertex_bases: int
+    n_ray_bases: int
+    kernel_ms: float
 
 
 class EnumerationSolver:
@@ -324,6 +342,29 @@ class EnumerationSolver:
                                          float(eps_opt), C.byref(cert)))
         self._cert, self._cert_basis = cert, [int(j) for j in basis]
         return cert
+
+    def costRanges(self, eps_opt: float = 1e-9, max_list: int = 0) -> CostRanges:
+        """Cost ranging of the optimum (enumgpu_cost_ranges): how far each c_j can move, all else fixed, before the
+        optimal vertex stops being optimal, exact at degenerate vertices (every feasible basis and every extreme ray
+        is looked at).  Enumerates first if nothing has been.  Runs on the current CUDA device.  Raises
+        RuntimeError("objective is unbounded") on an unbounded LP.  max_list: ranks held on the device (0 = 2^26)."""
+        res = self._res if self._res is not None else self.enumerate()
+        if res.status != _abi.OK:
+            raise RuntimeError("the problem has no feasible basic solution")
+        p = self._problem
+        ps = _problem_struct(p.GetConstraintsMatrix(), p.GetRightHandSide(), p.GetObjectiveCoefficients(), p.IsMaximization())
+        out = _abi.Ranging()
+        _check(lib().enumgpu_cost_ranges(C.byref(ps), C.byref(self._options()), C.byref(res), float(eps_opt), int(max_list),
+                                         C.byref(out)))
+        if out.status == _abi.CERT_UNBOUNDED:
+            raise RuntimeError("objective is unbounded")
+        r = out.range[: out.n]
+        return CostRanges(int(out.status),
+                          np.array([v.decrease for v in r]), np.array([v.increase for v in r]),
+                          np.array([v.decrease_rank for v in r], dtype=np.uint64),
+                          np.array([v.increase_rank for v in r], dtype=np.uint64),
+                          np.array([bool(v.decrease_ray) for v in r]), np.array([bool(v.increase_ray) for v in r]),
+                          int(out.n_vertex_bases), int(out.n_ray_bases), float(out.kernel_ms))
 
     def certificateBasis(self):
         """The columns (ascending) of the basis the certificate belongs to: the enumeration's optimal basis, or with
