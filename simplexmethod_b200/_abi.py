@@ -127,6 +127,23 @@ class Ranging(C.Structure):
     ]
 
 
+class RhsRange(C.Structure):
+    _fields_ = [
+        ("shadow_price", C.c_double), ("decrease", C.c_double), ("increase", C.c_double),
+        ("decrease_rank", C.c_uint64), ("increase_rank", C.c_uint64),
+    ]
+
+
+class RhsRanging(C.Structure):
+    _fields_ = [
+        ("status", C.c_int32), ("m", C.c_int32), ("n_tight", C.c_int32), ("n_launches", C.c_int32),
+        ("n_bases", C.c_uint64), ("n_singular", C.c_uint64),
+        ("kernel_ms", C.c_double),
+        ("tight", C.c_int32 * MAX_N),
+        ("range", RhsRange * MAX_M),
+    ]
+
+
 # every symbol include/enumgpu.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "enumgpu_version": (C.c_int, []),
@@ -174,6 +191,8 @@ SYMBOLS = {
                                             C.c_int32, C.c_uint64, C.POINTER(Result)]),
     "enumgpu_cost_ranges": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Result), C.c_double, C.c_uint64,
                                        C.POINTER(Ranging)]),
+    "enumgpu_rhs_ranges": (C.c_int, [C.POINTER(Problem), C.POINTER(Options), C.POINTER(Optimum), C.c_double,
+                                      C.POINTER(RhsRanging)]),
 }
 
 MAX_OBJECTIVES = 1 << 20

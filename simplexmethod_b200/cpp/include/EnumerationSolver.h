@@ -147,6 +147,16 @@ public:
         return rangesWith(&enumgpu_cost_ranges, eps_opt, max_list);
     }
 
+    // Right-hand-side ranging of the optimum of the last solve() (enumgpu_rhs_ranges, current device): for every row
+    // i, the allowable decrease and increase of b_i over which the dual values stay optimal, exact under dual
+    // degeneracy, with the shadow price y*_i and the basis that attains each limit.  The duals are those of
+    // enumgpu_certify_optimum, whatever setOptimalDuals says.  Throws std::runtime_error("objective is unbounded") on
+    // an unbounded LP.  eps_opt < 0: 1e-9.
+    const enumgpu_rhs_ranging& rhsRanges(double eps_opt = -1.0)
+    {
+        return rhsRangesWith(&enumgpu_certify_optimum, &enumgpu_rhs_ranges, eps_opt);
+    }
+
 private:
     void need() const { if (!solved_) throw std::logic_error("EnumerationSolver: solve() has not been called"); }
     using CertifyFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const int32_t*, double, enumgpu_certificate*);
@@ -186,6 +196,24 @@ private:
         if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
         if (ranging_.status == ENUMGPU_CERT_UNBOUNDED) throw std::runtime_error("objective is unbounded");
         return ranging_;
+    }
+    using OptimumFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const enumgpu_result*, double, uint64_t,
+                              enumgpu_optimum*);
+    using RhsRangesFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const enumgpu_optimum*, double,
+                                enumgpu_rhs_ranging*);
+    const enumgpu_rhs_ranging& rhsRangesWith(OptimumFn optimum, RhsRangesFn fn, double eps_opt)
+    {
+        need();
+        if (res_.status != ENUMGPU_OK) throw std::runtime_error("the problem has no feasible basic solution");
+        const enumgpu_problem p = problemStruct();
+        const enumgpu_options o = options();
+        enumgpu_optimum opt{};
+        int rc = optimum(&p, &o, &res_, eps_opt, 0, &opt);
+        if (rc == 0 && opt.cert.status == ENUMGPU_CERT_UNBOUNDED) throw std::runtime_error("objective is unbounded");
+        if (rc == 0) rc = fn(&p, &o, &opt, eps_opt, &rhs_ranging_);
+        if (rc == ENUMGPU_ERR_CUDA) throw std::runtime_error(std::string("libenumgpu: ") + enumgpu_last_error());
+        if (rc < 0) throw std::invalid_argument(std::string("libenumgpu: ") + enumgpu_last_error());
+        return rhs_ranging_;
     }
     static uint64_t binomial(int n, int k)          // C(n, k) for n <= 64, k <= 16: exact in 64 bits
     {
@@ -241,13 +269,12 @@ private:
     double eps_feas_ = -1.0, eps_piv_ = -1.0;
     uint64_t rank_begin_ = 0, rank_end_ = 0;
     CertifyFn check_unbounded_ = nullptr;      // &enumgpu_certify when setCheckUnbounded(true)
-    using OptimumFn = int (*)(const enumgpu_problem*, const enumgpu_options*, const enumgpu_result*, double, uint64_t,
-                              enumgpu_optimum*);
     OptimumFn optimal_duals_ = nullptr;        // &enumgpu_certify_optimum when setOptimalDuals(true)
     enumgpu_result res_{};
     std::vector<enumgpu_result> obj_res_;      // solveObjectives(), one per cost vector
     enumgpu_certificate cert_{};
     enumgpu_ranging ranging_{};
+    enumgpu_rhs_ranging rhs_ranging_{};
     std::vector<int> cert_basis_;
     int cert_source_ = ENUMGPU_OPT_WINNER;
     bool solved_ = false, certified_ = false;

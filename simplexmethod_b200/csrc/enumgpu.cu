@@ -21,6 +21,7 @@
 #include "k_shared.cuh"
 #include "k_objectives.cuh"
 #include "k_ranging.cuh"
+#include "k_rhs_ranging.cuh"
 
 using namespace enumgpu;
 
@@ -2213,6 +2214,141 @@ extern "C" int enumgpu_cost_ranges(const enumgpu_problem* p, const enumgpu_optio
     }
     if ((rc = require_device()) || (rc = cost_ranges_device(p, rs, rays ? &aux : nullptr, rsa, opt, eps_opt, max_list, out)))
         return out->status = rc;
+    return ENUMGPU_OK;
+}
+
+// ------------------------------------------------------------------ right-hand-side ranging (DESIGN.md §3.4)
+
+struct RhsLaunch {
+    const double* A;
+    const int32_t* J;
+    int n_tight, n;
+    const uint64_t* binom;
+    uint64_t total, total_full, rank_star;
+    double thr, rel_eps, eps_feas, eps_opt;
+    int rule;
+    Best* best;
+    unsigned long long* counters;
+};
+
+// The grid is the resident blocks that fill the device, or fewer when the runs of kRhsRun ranks are fewer; the block
+// count sizes `best`, so it comes back in *blocks.  a.best == nullptr: only the grid.
+template <int M>
+static cudaError_t launch_rhs(const RhsLaunch& a, int dev, cudaStream_t st, unsigned* blocks)
+{
+    if (!a.best) {
+        int sms = 148, per_sm = 1;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_rhs_ranging<M>, kRhsThreads, 0);
+        if (e != cudaSuccess) return e;
+        const uint64_t need = ((a.total + kRhsRun - 1) / kRhsRun + kRhsWarps - 1) / kRhsWarps;
+        *blocks = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>(need, (uint64_t)sms * std::max(per_sm, 1)));
+        return cudaSuccess;
+    }
+    k_rhs_ranging<M><<<*blocks, kRhsThreads, 0, st>>>(a.A, a.A + (size_t)M * a.n, a.J, a.n_tight, a.n, a.binom, a.total,
+                                                      a.total_full, a.rank_star, a.thr, a.rule, a.rel_eps, a.eps_feas,
+                                                      a.eps_opt, a.best, a.counters);
+    return cudaGetLastError();
+}
+
+static cudaError_t dispatch_rhs(int m, const RhsLaunch& a, int dev, cudaStream_t st, unsigned* blocks)
+{
+    switch (m) {
+#define ENUMGPU_CASE(M_) case M_: return launch_rhs<M_>(a, dev, st, blocks);
+        ENUMGPU_CASE(1) ENUMGPU_CASE(2) ENUMGPU_CASE(3) ENUMGPU_CASE(4)
+        ENUMGPU_CASE(5) ENUMGPU_CASE(6) ENUMGPU_CASE(7) ENUMGPU_CASE(8)
+        ENUMGPU_CASE(9) ENUMGPU_CASE(10) ENUMGPU_CASE(11) ENUMGPU_CASE(12)
+        ENUMGPU_CASE(13) ENUMGPU_CASE(14) ENUMGPU_CASE(15) ENUMGPU_CASE(16)
+#undef ENUMGPU_CASE
+    }
+    return cudaErrorInvalidValue;
+}
+
+// The device part of enumgpu_rhs_ranges: every m-subset of J (out->tight) in one launch, then the finish.
+static int rhs_ranges_device(const enumgpu_problem* p, const Resolved& rs, const enumgpu_optimum* dual, double eps_opt,
+                             enumgpu_rhs_ranging* out)
+{
+    const int m = p->m, n = p->n;
+    CallStream cs;
+    DeviceProblem D;
+    StreamBuf b_J, b_y, b_best, b_cnt, b_out;
+    const uint64_t* binom = nullptr;
+    int rc;
+    if ((rc = cs.open(true)) || (rc = upload_problem(p, cs.st, &D)) || (rc = device_binom(cs.dev, &binom))) return rc;
+    const cudaStream_t st = cs.st;
+    RhsLaunch a{D.dp.A_colmajor, nullptr, out->n_tight, n, binom, out->n_bases, rs.total, dual->rank,
+                pivot_threshold(rs, D.scale), rs.rule == ENUMGPU_PIVOT_RELATIVE ? rs.eps_piv : 0.0, rs.eps_feas, eps_opt,
+                rs.rule, nullptr, nullptr};
+    unsigned blocks = 0;
+    CU(dispatch_rhs(m, a, cs.dev, st, &blocks));
+    CU(b_J.alloc(sizeof(int32_t) * out->n_tight, st));
+    CU(b_y.alloc(sizeof(double) * m, st));
+    CU(b_best.alloc(sizeof(Best) * 2 * m * blocks, st));
+    CU(b_cnt.alloc(2 * sizeof(unsigned long long), st));
+    CU(b_out.alloc(sizeof(enumgpu_rhs_range) * m, st));
+    CU(cudaMemcpyAsync(b_J.p, out->tight, sizeof(int32_t) * out->n_tight, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(b_y.p, dual->cert.y, sizeof(double) * m, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(b_cnt.p, 0, 2 * sizeof(unsigned long long), st));
+    a.J = b_J.as<int32_t>();
+    a.best = b_best.as<Best>();
+    a.counters = b_cnt.as<unsigned long long>();
+    CU(cudaEventRecord(cs.e0, st));
+    CU(dispatch_rhs(m, a, cs.dev, st, &blocks));
+    k_rhs_ranging_finish<<<1, 32, 0, st>>>(b_best.as<Best>(), (int)blocks, m, b_y.as<double>(), b_out.as<enumgpu_rhs_range>());
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(cs.e1, st));
+    unsigned long long cnt[2] = {0, 0};
+    CU(cudaMemcpyAsync(out->range, b_out.p, sizeof(enumgpu_rhs_range) * m, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(cnt, b_cnt.p, sizeof cnt, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    out->kernel_ms = ms;
+    out->n_launches = 2;
+    out->n_singular = cnt[0];
+    if (cnt[1]) return fail(ENUMGPU_ERR_ARG, "rhs_ranges: the basis of dual is singular or infeasible under these options (dual came from other options)");
+    out->status = ENUMGPU_CERT_OPTIMAL;
+    return ENUMGPU_OK;
+}
+
+extern "C" int enumgpu_rhs_ranges(const enumgpu_problem* p, const enumgpu_options* o, const enumgpu_optimum* dual,
+                                  double eps_opt, enumgpu_rhs_ranging* out)
+{
+    g_err[0] = 0;
+    if (!out) return fail(ENUMGPU_ERR_ARG, "rhs_ranges: out is NULL");
+    memset(out, 0, sizeof *out);
+    if (o && (o->rank_begin != 0 || o->rank_end != 0))
+        return out->status = fail(ENUMGPU_ERR_ARG, "rhs_ranges: a rank range is not supported (the ranges are a statement about the whole space)");
+    if (o && (o->shard_index != 0 || o->shard_count != 0))
+        return out->status = fail(ENUMGPU_ERR_ARG, "rhs_ranges: shards are not supported");
+    const enumgpu_options oc = whole_space_options(o);
+    Resolved rs;
+    int rc = resolve(p, &oc, &rs, true);
+    if (rc) return out->status = rc;
+    const int m = p->m, n = p->n;
+    out->m = m;
+    int32_t S[kMaxM];
+    if (!dual || dual->cert.m != m || dual->cert.n != n || dual->cert.status < 0 || dual->rank >= rs.total ||
+        enumgpu_unrank(n, m, dual->rank, S) != 0 || memcmp(S, dual->basis, sizeof(int32_t) * m))
+        return out->status = fail(ENUMGPU_ERR_ARG, "rhs_ranges: dual is not an optimum of this LP (enumgpu_certify_optimum, m = %d, n = %d)", m, n);
+    if (dual->cert.status != ENUMGPU_CERT_OPTIMAL) {     // no dual-feasible y*: no ranges
+        out->status = dual->cert.status;
+        for (int i = 0; i < m; ++i) out->range[i] = enumgpu_rhs_range{NAN, NAN, NAN, UINT64_MAX, UINT64_MAX};
+        return ENUMGPU_OK;
+    }
+    eps_opt = resolve_eps_opt(eps_opt);
+    // J: the basis and every column whose reduced cost is tight at y*
+    for (int j = 0, k = 0; j < n; ++j) {
+        const bool basic = k < m && S[k] == j;
+        if (basic) ++k;
+        const double r = dual->cert.reduced_cost[j], rk = p->maximize ? -r : r;
+        if (basic || rk <= eps_opt) out->tight[out->n_tight++] = j;
+    }
+    out->n_bases = binom_mk(out->n_tight, m);
+    if ((rc = require_device()) || (rc = rhs_ranges_device(p, rs, dual, eps_opt, out))) {
+        out->status = rc;
+        return rc;
+    }
     return ENUMGPU_OK;
 }
 

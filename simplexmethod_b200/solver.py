@@ -175,6 +175,25 @@ class CostRanges(NamedTuple):
     kernel_ms: float
 
 
+class RhsRanges(NamedTuple):
+    """Right-hand-side ranging of EnumerationSolver.rhsRanges(): for each row i, b_i can fall by decrease[i] or rise
+    by increase[i] (np.inf: without limit) and the dual values stay optimal; over that interval the objective is
+    objective + delta * shadow_price[i].  *_rank[i] is the basis (a rank among the C(n, m) bases) that attains the
+    limit (UINT64_MAX: none).  tight: the columns whose reduced cost is tight at the duals, the basis included;
+    n_bases = C(len(tight), m) bases were looked at, n_singular of them singular.  status is CERT_OPTIMAL, or
+    CERT_BOUNDED / CERT_UNDECIDED when no dual-feasible basis was found (every range NaN)."""
+    status: int
+    shadow_price: np.ndarray
+    decrease: np.ndarray
+    increase: np.ndarray
+    decrease_rank: np.ndarray
+    increase_rank: np.ndarray
+    tight: list
+    n_bases: int
+    n_singular: int
+    kernel_ms: float
+
+
 class EnumerationSolver:
     """Solve a Canonical LP by enumerating all C(n, m) bases on the GPU(s).
 
@@ -365,6 +384,32 @@ class EnumerationSolver:
                           np.array([v.increase_rank for v in r], dtype=np.uint64),
                           np.array([bool(v.decrease_ray) for v in r]), np.array([bool(v.increase_ray) for v in r]),
                           int(out.n_vertex_bases), int(out.n_ray_bases), float(out.kernel_ms))
+
+    def rhsRanges(self, eps_opt: float = 1e-9) -> RhsRanges:
+        """Right-hand-side ranging of the optimum (enumgpu_rhs_ranges): how far each b_i can move, all else fixed,
+        while the dual values stay optimal, exact under dual degeneracy (every nonsingular basis of the tight columns
+        is looked at, feasible at b or not).  The duals are those of a dual-feasible optimal basis
+        (enumgpu_certify_optimum), whatever optimal_duals is set to.  Enumerates first if nothing has been.  Runs on
+        the current CUDA device.  Raises RuntimeError("objective is unbounded") on an unbounded LP."""
+        res = self._res if self._res is not None else self.enumerate()
+        if res.status != _abi.OK:
+            raise RuntimeError("the problem has no feasible basic solution")
+        p = self._problem
+        ps = _problem_struct(p.GetConstraintsMatrix(), p.GetRightHandSide(), p.GetObjectiveCoefficients(), p.IsMaximization())
+        o = self._options()
+        opt = _abi.Optimum()
+        _check(lib().enumgpu_certify_optimum(C.byref(ps), C.byref(o), C.byref(res), float(eps_opt), 0, C.byref(opt)))
+        if opt.cert.status == _abi.CERT_UNBOUNDED:
+            raise RuntimeError("objective is unbounded")
+        out = _abi.RhsRanging()
+        _check(lib().enumgpu_rhs_ranges(C.byref(ps), C.byref(o), C.byref(opt), float(eps_opt), C.byref(out)))
+        r = out.range[: out.m]
+        return RhsRanges(int(out.status), np.array([v.shadow_price for v in r]),
+                         np.array([v.decrease for v in r]), np.array([v.increase for v in r]),
+                         np.array([v.decrease_rank for v in r], dtype=np.uint64),
+                         np.array([v.increase_rank for v in r], dtype=np.uint64),
+                         [int(j) for j in out.tight[: out.n_tight]], int(out.n_bases), int(out.n_singular),
+                         float(out.kernel_ms))
 
     def certificateBasis(self):
         """The columns (ascending) of the basis the certificate belongs to: the enumeration's optimal basis, or with
